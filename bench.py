@@ -3,6 +3,8 @@
 
     python bench.py --gpus N --steps K --warmup W            (this repo's CUDA path)
     python bench.py --impl reference --gpus N --steps K ...   (CPU path: the oracle port, all host threads)
+    python bench.py --gpus 1 ... --dump-outputs DIR           (also writes the last timed step's result table as .npy files,
+                                                               for comparing two builds output for output)
 
 Workload (BASELINE.json configs[1], SURVEY.md section 8d): 50 M-read single sample, L = 75, NextSeq poly-G
 tails, ``-a illumina -nxt 20 -q 20``, all ordered libraries incl. a 100 000-entry mRNA library.  A step is
@@ -24,6 +26,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the bench writes nothing into the tree it runs from (which may be read-only)
 
 import numpy as np  # noqa: E402
 import torch  # noqa: E402
@@ -71,7 +74,13 @@ def parse_args():
     ap.add_argument("--exchange-unique", action="store_true",
                     help="N > 1, single-sample configs: local collapse + exchange of the unique sequences instead of sharding before the collapse")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/<name>.npy (float64 / float32, < 64 MB in all)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
     c = CONFIG_TABLE[a.config]
     a.reads = a.reads or c["reads"]
     a.samples = a.samples or c["samples"]
@@ -315,7 +324,7 @@ def run_ingest_gz_guarded(fastq: np.ndarray, threads: int, timeout_s: int = 240)
         code = ("import sys, json, numpy as np; sys.path.insert(0, %r); import bench; "
                 "print('INGEST_GZ ' + json.dumps(bench.run_ingest_gz(np.fromfile(sys.argv[1], dtype=np.uint8), int(sys.argv[2]))))" % ROOT)
         try:
-            p = subprocess.run([sys.executable, "-c", code, unit, str(int(threads))], capture_output=True, text=True, timeout=timeout_s)
+            p = subprocess.run([sys.executable, "-B", "-c", code, unit, str(int(threads))], capture_output=True, text=True, timeout=timeout_s)
         except subprocess.TimeoutExpired:
             return {"error": "timed out after %d s" % timeout_s}
         for ln in p.stdout.splitlines():
@@ -373,6 +382,63 @@ def run_dropin(args, dev, lset, libs, fq_dev, cfg_id):
         shutil.rmtree(tmp, ignore_errors=True)
 
 
+DUMP_KEYS = 1 << 16  # unique sequences in the sample that --dump-outputs writes row by row
+DUMP_ROW_BYTES = 48 << 20  # bound of that sample's rows (text, counts, annotation); the whole-table files add 88 bytes per sample
+
+
+def sample_fastq(libs, cfg_id, gs, n_reads, multi_sample, device):
+    """FASTQ bytes of global sample ``gs`` of the workload, on ``device``: seeded, identical from run to run."""
+    import dataclasses
+
+    from mirge_b200 import synth
+
+    rc = dataclasses.replace(synth.CONFIGS[cfg_id], sample_seed=gs if multi_sample else 0)
+    gen = synth.ReadGenerator(libs, rc, device)
+    gen.gen.manual_seed(2000 + cfg_id + 7919 * gs)
+    return gen.fastq(n_reads, first_index=gs * n_reads)
+
+
+def dump_outputs(out_dir, tab, columns, annot, hit, n_reads):
+    """--dump-outputs: the result table of a pass -- unique sequences, their per-sample counts, their annotation -- as .npy
+    files.  Whole-table totals, plus every column for a fixed, seeded sample of the sequences taken in bytewise order of
+    their text (key ids follow the insertion order of concurrent threads and differ from run to run).
+      totals            [reads, unique sequences, annotated sequences]
+      keys_per_round    [11]     sequences annotated in round 0..9, last: unannotated
+      reads_per_round   [S, 11]  counts of those sequences per sample (the numbers of annotation.report.csv)
+      sample_sequences  [K, W]   ASCII codes of the sampled sequences, 0-padded (float32)
+      sample_counts     [K, S]   their counts per sample
+      sample_annotation [K, 4]   their round (255: none), mismatches, library entry and offset of the hit"""
+    from mirge_b200.manifoldAlign import decode_hits
+
+    os.makedirs(out_dir, exist_ok=True)
+    n = int(tab.n_keys)
+    dev = annot.device
+    counts = torch.zeros(len(columns), n, dtype=torch.float64, device=dev)
+    for s, (ids, cnt) in enumerate(columns):
+        counts[s, ids.long()] = cnt.double()
+    rnd = annot[:n].long().clamp(max=10)  # rounds are 0..9; 0xFF (unannotated) -> 10
+    reads_per_round = torch.zeros(len(columns), 11, dtype=torch.float64, device=dev).index_add_(1, rnd, counts)
+    perm, offsets, data = tab.export_sorted_device()
+    lens_all = offsets[1:] - offsets[:-1]
+    width = max(int(lens_all.max().item()), 1) if n else 1
+    k = min(n, DUMP_KEYS, DUMP_ROW_BYTES // (4 * width + 8 * len(columns) + 8 * 4))
+    pos = torch.from_numpy(np.sort(np.random.default_rng(20240).choice(n, k, replace=False))).to(dev)
+    sel, lo, lens = perm[pos], offsets[pos], lens_all[pos]
+    col = torch.arange(width, device=dev)
+    text = torch.where(col < lens[:, None], data[(lo[:, None] + col).clamp(max=data.numel() - 1)], 0)
+    rounds, mm, ref, off = decode_hits(annot[sel].cpu().numpy(), hit[sel].cpu().numpy())
+    out = {
+        "totals": np.array([n_reads, n, int((rnd < 10).sum().item())], dtype=np.float64),
+        "keys_per_round": torch.bincount(rnd, minlength=11).double().cpu().numpy(),
+        "reads_per_round": reads_per_round.cpu().numpy(),
+        "sample_sequences": text.float().cpu().numpy(),
+        "sample_counts": counts[:, sel].T.contiguous().cpu().numpy(),
+        "sample_annotation": np.stack([rounds, mm, ref, off], axis=1).astype(np.float64),
+    }
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def run_b200(args):
     import torch.distributed as dist
 
@@ -388,6 +454,8 @@ def run_b200(args):
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
     if world > 1:
+        if args.dump_outputs:
+            raise SystemExit("bench: --dump-outputs writes the table of one process; run it with one GPU")
         dist.init_process_group("nccl", device_id=torch.device("cuda", local))
     dev = D.Device(local)
     torch.cuda.set_device(dev.tdev)
@@ -400,17 +468,8 @@ def run_b200(args):
     cfg = synth.trim_config_for(cfg_id, args.count_mode)
     eng = D.DigestEngine(dev, cfg)
     umi = cfg.umi()
-    import dataclasses
-
     # this GPU's samples (C4: per-sample abundance perturbation, synth.ReadConfig.sample_seed); resident in HBM
-    fqs = []
-    for s_i in range(args.samples):
-        gs = rank * args.samples + s_i  # global sample index
-        rc = dataclasses.replace(synth.CONFIGS[cfg_id], sample_seed=gs if args.samples > 1 else 0)
-        gen = synth.ReadGenerator(libs, rc, dev.tdev)
-        gen.gen.manual_seed(2000 + cfg_id + 7919 * gs)
-        fqs.append(gen.fastq(args.reads, first_index=gs * args.reads))
-        del gen
+    fqs = [sample_fastq(libs, cfg_id, rank * args.samples + s_i, args.reads, args.samples > 1, dev.tdev) for s_i in range(args.samples)]
     rc = synth.CONFIGS[cfg_id]
     torch.cuda.synchronize()
     nbytes = int(sum(f.numel() for f in fqs))
@@ -522,6 +581,9 @@ def run_b200(args):
     e1.record()
     barrier()
     torch.cuda.profiler.stop()
+    launches = (dev.launches - launches0) // max(args.steps, 1)
+    if args.dump_outputs:  # the last timed step's table (before the trace step and the e2e leg, which reuse it)
+        dump_outputs(args.dump_outputs, state["tab"], state["columns"], state["annot"], state["hit"], n_rec)
     trace_to = os.environ.get("MIRGE_B200_TRACE")
     if trace_to and rank == 0:
         # diagnostics, outside the timed region: one more step under torch.profiler, kernels / copies per stream in time order
@@ -544,7 +606,6 @@ def run_b200(args):
     timers = dev.timer_totals()
     dev.timing = False
     stats = dict(eng.stats)
-    launches = (dev.launches - launches0) // max(args.steps, 1)
     clk = clocks.stop() if clocks else None
     tms = torch.tensor([ms], device=dev.tdev, dtype=torch.float64)
     if world > 1:

@@ -175,7 +175,9 @@ def _reference_baking():
         m = pytest.importorskip(mod)
         if not getattr(m, "__file__", None):
             pytest.skip("%s in sys.modules is a stand-in" % mod)
-    ref = "/root/reference"
+    from tests.golden.make_reference_golden import REFERENCE
+
+    ref = str(REFERENCE)
     if os.path.isdir(os.path.join(ref, "mirge")) and ref not in sys.path:
         sys.path.append(ref)
     try:
