@@ -405,6 +405,19 @@ int mirge_annotate_allhits(mirge_ctx *ctx, const mirge_library *lib, const mirge
                            const mirge_table *t, const uint32_t *d_ids, uint64_t n_ids, const uint64_t *d_hit,
                            int fill, uint32_t *d_counts, const uint64_t *d_offs, uint64_t *d_out, void *stream);
 
+/* The per-round SAM records of -bam / -trf (manifoldAlign.py:20-62), one per (d_ids[i], d_hits[i]) pair: key id of
+ * table t and hit word of `policy`'s round against `lib`.  Record i is
+ *   QNAME \t 0 \t RNAME \t POS \t 255 \t <n>M \t * \t 0 \t 0 \t SEQ \t QUAL \t XA:i:<x> \t MD:Z:<md> \t NM:i:<nm> \n
+ * QNAME = the key text; SEQ = the round's query (trailing T run stripped with strip_polyT, then trim5 / trim3), n its
+ * length, QUAL n x 'I'; RNAME = d_names[d_name_off[r] .. d_name_off[r + 1]) of r = MIRGE_HIT_REF; POS = offset + 1;
+ * MD / NM over the reference text (ambiguous bases print as 'N'), XA = mismatches inside the seed (seed_len, 0 = all).
+ * Two calls: fill = 0 writes d_lens[i] = bytes of record i; after an exclusive scan into d_offs, fill = 1 writes the
+ * records to d_out + d_offs[i]. */
+int mirge_sam_format(mirge_ctx *ctx, const mirge_library *lib, const mirge_round_policy *policy, const mirge_table *t,
+                     const uint32_t *d_ids, const uint64_t *d_hits, uint64_t n, const uint8_t *d_names,
+                     const uint64_t *d_name_off, int fill, uint32_t *d_lens, const uint64_t *d_offs, uint8_t *d_out,
+                     void *stream);
+
 /* ---- stage 4: counters of annotation.report.csv (summarize, summary.py:692-698,716-770) ---- */
 /* For every (key id, count) pair of ONE sample (the output of mirge_table_drain):
  *   d_round_sum[round of the key] += count            (u64[10]; unannotated keys are skipped)

@@ -765,25 +765,89 @@ def fill_annotation(pdDataFrame, annot_all, ref_all, order, names_of, spike: boo
     return pdDataFrame.fillna("")
 
 
+def owner_sam_records(dev, libs, keys, annot, hit_d, rounds):
+    """The SAM records of the sequences a rank owns for the (round, file) pairs ``rounds`` (manifoldAlign.sam_rounds),
+    formatted on its GPU: [record bytes uint8, record lengths int64, owner key id int64, round uint8], records grouped
+    by round, key ids ascending inside a round and, inside a sequence, in the order bowtie prints them."""
+    import numpy as np
+
+    from . import manifoldAlign as MA
+    from .libraries import ROUND_LIBS, round_policies
+
+    pols = round_policies()
+    data, lens, ids, rnds = [], [], [], []
+    for rnd, _ in rounds:
+        own = np.nonzero(annot == rnd)[0]
+        if own.size == 0:
+            continue
+        lib = libs[ROUND_LIBS[rnd]]
+        rec_ids, rec_hits = MA.round_sam_pairs(dev, lib, pols[rnd], keys, own, hit_d)
+        for chunk, n in MA.sam_records(dev, lib, pols[rnd], keys, rec_ids, rec_hits):
+            data.append(chunk)
+            lens.append(n)
+        ids.append(rec_ids)
+        rnds.append(np.full(rec_ids.size, rnd, dtype=np.uint8))
+    cat = lambda parts, dt: np.concatenate(parts).astype(dt, copy=False) if parts else np.zeros(0, dtype=dt)
+    return [cat(data, np.uint8), cat(lens, np.int64), cat(ids, np.int64), cat(rnds, np.uint8)]
+
+
+def write_gathered_sam(workDir, gathered, rounds, order, offs, n_all, batch: int = 1 << 20):
+    """Rank 0: the owners' SAM records (per rank, what owner_sam_records returned) appended to the per-round files in the
+    order the single-process bwtAlign writes them: file by file in round order, table rows ascending, a sequence's
+    records in their owner's order.  Records of sequences that are not a row of the table (no sample counted them,
+    assemble_table) are dropped.  Returns (records, bytes) written."""
+    import os
+
+    import numpy as np
+
+    row_of = np.full(n_all, -1, dtype=np.int64)
+    row_of[order] = np.arange(order.size, dtype=np.int64)
+    data = np.concatenate([g[0] for g in gathered])
+    lens = np.concatenate([g[1] for g in gathered])
+    rows = np.concatenate([row_of[offs[r] + g[2]] for r, g in enumerate(gathered)])
+    rnds = np.concatenate([g[3] for g in gathered])
+    start = np.cumsum(lens) - lens
+    n_rec = n_bytes = 0
+    for rnd, fname in rounds:
+        sel = np.nonzero((rnds == rnd) & (rows >= 0))[0]
+        if sel.size == 0:
+            continue
+        sel = sel[np.argsort(rows[sel], kind="stable")]
+        with open(os.path.join(str(workDir), fname), "ab") as fh:
+            for b in range(0, sel.size, batch):
+                s = sel[b : b + batch]
+                ln = lens[s]
+                at = np.cumsum(ln) - ln
+                src = np.repeat(start[s] - at, ln) + np.arange(int(ln.sum()), dtype=np.int64)
+                fh.write(memoryview(data[src]))
+                n_bytes += int(ln.sum())
+        n_rec += int(sel.size)
+    return n_rec, n_bytes
+
+
 def bwtAlign_sharded(args, pdDataFrame, workDir, ref_db, libraries=None, group=None):
     """Call on every rank after baking_sharded (pdDataFrame: its result on rank 0, None elsewhere).  Every rank
-    annotates the sequences it owns; rank 0 returns the DataFrame manifoldAlign.bwtAlign would return."""
+    annotates the sequences it owns; rank 0 returns the DataFrame manifoldAlign.bwtAlign would return.  With -bam /
+    -trf every rank formats the SAM records of its own sequences and rank 0 writes the per-round files, the same bytes
+    the single-process bwtAlign writes; the other ranks write nothing."""
     import numpy as np
 
     from . import manifoldAlign as MA
     from .libraries import ROUND_LIBS
 
-    if getattr(args, "bam_out", False) or getattr(args, "tRNA_frag", False):
-        raise RuntimeError("-bam / -trf are written by the single-process bwtAlign only")
     rank, world = dist.get_rank(group), dist.get_world_size(group)
     dev, owner = _SHARD["dev"], _SHARD["owner"]
     libs = libraries or MA.load_libraries(args, ref_db, dev)
     spike = bool(getattr(args, "spikeIn", False))
-    annot_d, hit_d = MA.annotate_keys(dev, libs, MA.KeySet.from_table(owner), spike)
+    keys = MA.KeySet.from_table(owner)
+    annot_d, hit_d = MA.annotate_keys(dev, libs, keys, spike)
     annot = annot_d.cpu().numpy()
     _, _mm, ref, _off = MA.decode_hits(annot, hit_d.cpu().numpy())
     # round and reference index of every owned sequence at rank 0; the names are looked up there (libraries are replicated)
-    gathered = gather_arrays([annot.astype(np.uint8), ref.astype(np.int64)], 0, group, dev.tdev if "nccl" in str(dist.get_backend(group)) else None)
+    tdev = dev.tdev if "nccl" in str(dist.get_backend(group)) else None
+    gathered = gather_arrays([annot.astype(np.uint8), ref.astype(np.int64)], 0, group, tdev)
+    rounds = MA.sam_rounds(args, spike)
+    sam = gather_arrays(owner_sam_records(dev, libs, keys, annot, hit_d, rounds), 0, group, tdev) if rounds else None
     if rank != 0:
         return None
     if _SHARD["n_all"]:
@@ -791,5 +855,7 @@ def bwtAlign_sharded(args, pdDataFrame, workDir, ref_db, libraries=None, group=N
         ref_all = np.concatenate([g[1] for g in gathered])
     else:
         annot_all, ref_all = np.zeros(0, dtype=np.uint8), np.zeros(0, dtype=np.int64)
+    if sam is not None:
+        write_gathered_sam(workDir, sam, rounds, _SHARD["order"], _SHARD["offs"], _SHARD["n_all"])
     names_of = {rnd: libs[ROUND_LIBS[rnd]].names for rnd in range(10 if spike else 9)}
     return fill_annotation(pdDataFrame, annot_all, ref_all, _SHARD["order"], names_of, spike)

@@ -113,7 +113,6 @@ class DeviceLibrary:
             raise MirgeError("library %s too large for 32-bit positions" % key)
         if len(lens) and int(lens.max()) >= (1 << 28):
             raise MirgeError("library %s has a reference longer than 2^28 bases" % key)
-        self.ref_off_host = off
         self.max_ref_len = int(lens.max()) if len(lens) else 0
         self.ref_off = torch.from_numpy(off.astype(np.uint32).view(np.int32)).to(dev.tdev)
         text = torch.frombuffer(bytearray(b"".join(seqs)), dtype=torch.uint8).to(dev.tdev) if self.n_bases else \
@@ -132,19 +131,6 @@ class DeviceLibrary:
         off_d = torch.from_numpy(off).to(dev.tdev)
         self.ref_block = (torch.searchsorted(off_d, starts, right=True) - 1).clamp_(0, max(self.n_refs - 1, 0)).to(torch.int32)
         self._build_index()
-
-    def host_text(self) -> np.ndarray:
-        """ASCII text of the concatenated references on the host (decoded once from the device copy; only the SAM
-        writers need it, for MD:Z tags)."""
-        if getattr(self, "_host_text", None) is None:
-            words = self.packed[: (self.n_bases + 15) // 16].cpu().numpy().view(np.uint32)
-            codes = ((words[:, None] >> (2 * np.arange(16, dtype=np.uint32))) & 3).astype(np.uint8).reshape(-1)[: self.n_bases]
-            text = np.frombuffer(b"ACGT", dtype=np.uint8)[codes]
-            nm = self.nmask.cpu().numpy().view(np.uint32)
-            isn = ((nm[:, None] >> np.arange(32, dtype=np.uint32)) & 1).astype(bool).reshape(-1)[: self.n_bases]
-            text[isn] = ord("N")
-            self._host_text = text
-        return self._host_text
 
     def _base_struct(self) -> abi.Library:
         return abi.Library(self.packed.data_ptr(), self.nmask.data_ptr(), self.ref_off.data_ptr(), self.n_refs, self.n_bases,

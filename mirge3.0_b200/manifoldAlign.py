@@ -240,6 +240,17 @@ _SAM_BAM = {0: "miRge3_miRNA.sam", 8: "miRge3_miRNA.sam", 1: "miRge3_hairpin_miR
 _SAM_TRF = {2: "miRge3_tRNA.sam", 3: "miRge3_pre_tRNA.sam"}
 
 
+def sam_rounds(args, spike: bool):
+    """(round, SAM file name) of the rounds whose records the flags ask for, in the order they are appended."""
+    want_bam, want_trf = bool(getattr(args, "bam_out", False)), bool(getattr(args, "tRNA_frag", False))
+    out = []
+    for rnd in range(10 if spike else 9):
+        fname = (_SAM_BAM.get(rnd) if want_bam else None) or (_SAM_TRF.get(rnd) if want_trf else None)
+        if fname is not None:
+            out.append((rnd, fname))
+    return out
+
+
 def best_stratum_hits(dev: Device, lib, pol, keys: KeySet, ids: np.ndarray, hit_d: torch.Tensor):
     """All hits of the best stratum for the sequences ``ids`` of a -a --best --strata round: (row index into ids,
     hit word) pairs, unique, grouped by row, ascending hit word inside a row."""
@@ -292,21 +303,81 @@ def round_query_text(seq: str, pol) -> str:
     return q[pol.trim5 : max(len(q) - pol.trim3, pol.trim5)]
 
 
-def write_round_sam(path, seqs, rows: np.ndarray, hits: np.ndarray, lib, pol):
-    """Append bowtie-format SAM records (one per (row, hit word) pair, in the given order) to ``path``."""
-    text = lib.host_text()
-    off_h = lib.ref_off_host
-    with open(path, "a+") as fh:
-        for row, h in zip(rows.tolist(), hits.tolist()):
-            ref, off = (h >> 28) & 0xFFFFFFF, h & 0xFFFFFFF
-            name = seqs[row]
-            q = round_query_text(name, pol)
-            a = int(off_h[ref]) + off
-            seg = text[a : a + len(q)].tobytes().decode("latin-1")
-            seed = len(q) if pol.seed_len == 0 else min(pol.seed_len, len(q))
-            xa, md, nm = _md_tag(q, seg, seed)
-            fh.write("%s\t0\t%s\t%d\t255\t%dM\t*\t0\t0\t%s\t%s\tXA:i:%d\tMD:Z:%s\tNM:i:%d\n"
-                     % (name, lib.names[ref], off + 1, len(q), q, "I" * len(q), xa, md, nm))
+SAM_SLICE_BYTES = 512 << 20  # device buffer of one fill launch of mirge_sam_format; a larger round is formatted in slices
+
+
+def round_sam_pairs(dev: Device, lib, pol, keys: KeySet, ids: np.ndarray, hit_d: torch.Tensor):
+    """(key id, hit word) of every SAM record of one round for the sequences ``ids`` (key ids of ``keys``, in the order
+    the records are wanted), in the order bowtie prints them: the canonical hit of a -n / -v round; every hit of the best
+    stratum of a -a round (2, 3), hit words descending inside a sequence so that the canonical pick comes last (the
+    record the reference's parser keeps, manifoldAlign.py:50-56).  Returns (key ids int64 numpy, hit words int64 on the
+    device)."""
+    ids = np.asarray(ids, dtype=np.int64)
+    if pol.round in _SAM_TRF:
+        r_idx, words = best_stratum_hits(dev, lib, pol, keys, ids, hit_d)
+        o = np.lexsort((np.iinfo(np.int64).max - words.astype(np.int64), r_idx))  # sequence ascending, hit descending
+        return ids[r_idx[o]], torch.from_numpy(np.ascontiguousarray(words[o]).view(np.int64)).to(dev.tdev)
+    return ids, hit_d[torch.from_numpy(ids).to(dev.tdev)]
+
+
+def _sam_names(dev: Device, lib):
+    """The library's reference names on the device (bytes back to back, int64 offsets), made once per library."""
+    got = getattr(lib, "_sam_names", None)
+    if got is None:
+        enc = [nm.encode("utf-8") for nm in lib.names]
+        off = np.zeros(len(enc) + 1, dtype=np.int64)
+        np.cumsum(np.fromiter((len(b) for b in enc), dtype=np.int64, count=len(enc)), out=off[1:])
+        blob = torch.from_numpy(np.frombuffer(b"".join(enc) or b"\0", dtype=np.uint8).copy()).to(dev.tdev)
+        got = lib._sam_names = (blob, torch.from_numpy(off).to(dev.tdev))
+    return got
+
+
+def sam_records(dev: Device, lib, pol, keys: KeySet, ids: np.ndarray, hits_d: torch.Tensor, slice_bytes: int = 0):
+    """The bowtie SAM records of the (key id, hit word) pairs (ids[i], hits_d[i]), formatted on the device by
+    mirge_sam_format (csrc/sam_format.cuh) in that order.  Yields (record bytes uint8, record lengths int64) on the
+    host per slice of at most ``slice_bytes`` (SAM_SLICE_BYTES) bytes -- one record more when a single record is
+    larger."""
+    n = int(len(ids))
+    if n == 0:
+        return
+    ids_d = torch.from_numpy(np.asarray(ids).astype(np.int32)).to(dev.tdev)
+    hits_d = hits_d.to(torch.int64).contiguous()
+    names, name_off = _sam_names(dev, lib)
+    call = lambda fill, i0, i1, lens, offs, out: dev.check(dev.lib.mirge_sam_format(
+        dev.ctx, C.byref(lib.struct), C.byref(pol), C.byref(keys.struct), _ptr(ids_d[i0:i1]), _ptr(hits_d[i0:i1]), i1 - i0,
+        _ptr(names), _ptr(name_off), fill, _ptr(lens), _ptr(offs), _ptr(out), dev.stream()))
+    lens = dev.empty(n, torch.int32)
+    with dev.timed("sam_format"):
+        call(0, 0, n, lens, None, None)
+    dev.launches += 1
+    lens64 = lens[:n].to(torch.int64)
+    ends = torch.cumsum(lens64, 0)
+    ends_h, lens_h = ends.cpu().numpy(), lens64.cpu().numpy()
+    budget = int(slice_bytes or SAM_SLICE_BYTES)
+    i0 = 0
+    while i0 < n:
+        base = int(ends_h[i0 - 1]) if i0 else 0
+        i1 = max(i0 + 1, int(np.searchsorted(ends_h, base + budget, side="right")))
+        out = dev.empty(int(ends_h[i1 - 1]) - base, torch.uint8)
+        offs = ends[i0:i1] - lens64[i0:i1] - base
+        with dev.timed("sam_format"):
+            call(1, i0, i1, None, offs, out)
+        dev.launches += 1
+        yield out[: int(ends_h[i1 - 1]) - base].cpu().numpy(), lens_h[i0:i1]
+        i0 = i1
+
+
+def write_round_sam(path, dev: Device, lib, pol, keys: KeySet, ids: np.ndarray, hit_d: torch.Tensor, slice_bytes: int = 0):
+    """Append the SAM records of one round (round_sam_pairs of the sequences ``ids``, in that order) to ``path``; the
+    records are formatted on the device and copied to the host once per slice.  Returns (records, bytes) written."""
+    rec_ids, rec_hits = round_sam_pairs(dev, lib, pol, keys, ids, hit_d)
+    n_rec = n_bytes = 0
+    with open(path, "ab") as fh:
+        for chunk, lens in sam_records(dev, lib, pol, keys, rec_ids, rec_hits, slice_bytes):
+            fh.write(memoryview(chunk))
+            n_rec += int(lens.size)
+            n_bytes += int(chunk.size)
+    return n_rec, n_bytes
 
 
 def _filled_column(old: "pd.Series", rows: np.ndarray, names: np.ndarray, ref: np.ndarray):
@@ -434,10 +505,9 @@ def bwtAlign(args, pdDataFrame, workDir, ref_db, libraries: Optional[LibrarySet]
     libs = libraries or load_libraries(args, ref_db, dev)
     spike = bool(getattr(args, "spikeIn", False))
     annot_dv = hit_dv = None
-    seqs = None  # the index as Python strings: only where needed (a frame that did not come from baking(), SAM files)
     cached = pdDataFrame.attrs.get("_mirge_b200_keys")
     if cached is not None and getattr(cached.table, "dev", None) is dev and len(cached.order) == len(pdDataFrame) and \
-            not (getattr(args, "bam_out", False) or getattr(args, "tRNA_frag", False)) and _rows_match(cached, pdDataFrame.index):
+            _rows_match(cached, pdDataFrame.index):
         # the DataFrame comes straight from baking(): its packed keys are still on the device (row i = key id order[i])
         table, order = cached.table, cached.order
         keys = KeySet.from_table(table)
@@ -448,12 +518,14 @@ def bwtAlign(args, pdDataFrame, workDir, ref_db, libraries: Optional[LibrarySet]
         annot_dv, hit_dv = annot_all[sel], hit_all[sel]
         annot = annot_dv.cpu().numpy()
         hit = None  # (copied only if the columns have to be built on the host)
+        key_of_row, hit_of_key = order, hit_all
     else:
         seqs = pdDataFrame.index.to_numpy()
         keys = KeySet.from_strings(dev, list(seqs))
         annot_d, hit_d = annotate_keys(dev, libs, keys, spike)
         annot = annot_d.cpu().numpy()
         hit = hit_d.cpu().numpy()
+        key_of_row, hit_of_key = None, hit_d  # key id = row
     colnames = list(pdDataFrame.columns)
     n_rounds = 10 if spike else 9
     on_device = False
@@ -468,28 +540,14 @@ def bwtAlign(args, pdDataFrame, workDir, ref_db, libraries: Optional[LibrarySet]
     flag[annot != 0xFF] = 1
     pdDataFrame[colnames[0]] = flag
     # per-round SAM files for bamFmt.bow2bam (-bam) and the tRF block of summarize (-trf): records in the order
-    # bowtie prints them (input order = table order); -a rounds list every hit of the best stratum, the
-    # canonical pick last (the record the reference's parser keeps, manifoldAlign.py:50-56)
-    want_bam, want_trf = bool(getattr(args, "bam_out", False)), bool(getattr(args, "tRNA_frag", False))
-    if want_bam or want_trf:
-        pols = round_policies()
-        if seqs is None:
-            seqs = pdDataFrame.index.to_numpy()
-        for rnd in range(10 if spike else 9):
-            fname = (_SAM_BAM.get(rnd) if want_bam else None) or (_SAM_TRF.get(rnd) if want_trf else None)
-            if fname is None:
-                continue
-            rows = np.nonzero(annot == rnd)[0]
-            if rows.size == 0:
-                continue
-            lib = libs[ROUND_LIBS[rnd]]
-            if rnd in _SAM_TRF:
-                r_idx, words = best_stratum_hits(dev, lib, pols[rnd], keys, rows, hit_d)
-                order = np.lexsort((np.iinfo(np.int64).max - words.astype(np.int64), r_idx))  # row ascending, hit descending
-                sam_rows, sam_hits = rows[r_idx[order]], words[order]
-            else:
-                sam_rows, sam_hits = rows, hit[rows].view(np.uint64)
-            write_round_sam(Path(workDir) / fname, seqs, sam_rows, sam_hits, lib, pols[rnd])
+    # bowtie prints them (input order = table order, round_sam_pairs inside a sequence), formatted on the device
+    pols = round_policies()
+    for rnd, fname in sam_rounds(args, spike):
+        rows = np.nonzero(annot == rnd)[0]
+        if rows.size == 0:
+            continue
+        ids = rows if key_of_row is None else key_of_row[rows]
+        write_round_sam(Path(workDir) / fname, dev, libs[ROUND_LIBS[rnd]], pols[rnd], keys, ids, hit_of_key)
     finish = time.perf_counter()
     if not spike:
         pdDataFrame = pdDataFrame.drop(columns=["spike-in"])
