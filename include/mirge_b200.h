@@ -37,7 +37,7 @@
 extern "C" {
 #endif
 
-#define MIRGE_ABI_VERSION 3
+#define MIRGE_ABI_VERSION 4
 
 #define MIRGE_OK 0
 #define MIRGE_ERR_CUDA (-1)     /* CUDA runtime error (message has the cudaError string) */
@@ -249,31 +249,10 @@ int mirge_trim(mirge_ctx *ctx, const uint8_t *d_fastq, uint64_t nbytes, const ui
                uint64_t keys_capacity_words, uint64_t *d_trim_ctrl, void *d_scratch, uint64_t *d_ins,
                uint64_t ins_capacity, void *stream);
 
-/* ---- stages 1a + 1b in one pass: fused tokeniser + trim (the product path) -------------------------------------
- * The same result as mirge_tokenise_sync + mirge_line_index + mirge_trim without a separate pass over the bytes: a
- * persistent kernel takes the stream tile by tile through the bulk-copy engine (cp.async.bulk + mbarrier), finds the
- * line breaks of each tile in shared memory, numbers the records by a single-pass look-back over the tiles in front
- * and runs stage 1 of the split pipeline on the bytes where they lie; stages 2 / 3 and the whole-pipeline pass follow
- * as in mirge_trim.  Applies when mirge_digest_fused_ok() (3' adapters of <= 32 nt with indels, no qiagen UMIs,
- * automatic kernel choice); otherwise use the three calls above.
- * The number of records is not known beforehand: n_cap is the caller's bound (outputs and lists are sized by it:
- * d_line_start u32[4 n_cap + 4] or NULL, d_win / d_key_off for n_cap x slots or NULL, d_ins >= n_cap x slots
- * entries, d_scratch = mirge_digest_scratch_bytes(nbytes, n_cap)).  d_trim_ctrl (16 x u64, zeroed by the caller) as
- * for mirge_trim, plus [9] line breaks of the batch (with is_final, a last line without '\n' counts as complete),
- * [10] offset just behind the last complete record, relative to d_fastq rounded down to 16 bytes,
- * [2] bit 16: more than n_cap records -- repeat with n_cap >= [9] / 4; [2] bit 8: too many records for the
- * whole-pipeline list -- use the three-call path for this batch. */
-int mirge_digest_fused_ok(const mirge_ctx *ctx);
-uint64_t mirge_digest_scratch_bytes(uint64_t nbytes, uint64_t n_cap);
-int mirge_digest_tiles(mirge_ctx *ctx, const uint8_t *d_fastq, uint64_t nbytes, int is_final, uint64_t n_cap,
-                       uint32_t *d_line_start, uint16_t *d_win, uint32_t *d_key_off, uint32_t *d_keys,
-                       uint64_t keys_capacity_words, uint64_t *d_trim_ctrl, void *d_scratch, uint64_t *d_ins,
-                       uint64_t ins_capacity, void *stream);
-
 /* Kernel selection for mirge_trim: 0 = automatic (split bit-parallel pipeline when every adapter is a 3'
  * adapter with indels and <= 32 nt, else the generic full-DP kernel), 1 = always generic, 2 = bit-parallel
- * kernel without the split (one kernel + second pass; kept for the parity tests).  When the generic-free
- * path meets a record group that does not fit its shared-memory staging the group goes to the second pass. */
+ * kernel without the split (one kernel + second pass; kept for the parity tests).  When a bit-parallel kernel
+ * meets a record group that does not fit its shared-memory staging, the group goes to the second pass. */
 int mirge_trim_mode(mirge_ctx *ctx, int mode);
 
 /* ---- stage 2: collapse (digest.py:141-163,164-205,237-245) --------------------------------- */
@@ -286,13 +265,10 @@ int mirge_table_reset(mirge_ctx *ctx, const mirge_table *t, void *stream);
  * chain of dependent accesses of an insert). */
 int mirge_collapse_insert_list(mirge_ctx *ctx, const mirge_table *t, const uint32_t *d_keys, const uint64_t *d_ins,
                                uint64_t n_items, uint32_t *d_scratch, void *stream);
-/* Merge (key, count) records: d_rec = [count][key words...] back to back, d_rec_off[i] = word
- * offset of record i.  Used by the owner side of the hash-partitioned exchange. */
-int mirge_collapse_merge(mirge_ctx *ctx, const mirge_table *t, const uint32_t *d_rec,
-                         const uint32_t *d_rec_off, uint64_t n_rec, uint32_t *d_deferred, void *stream);
-/* The same when the records were received straight into the table's arena (the all-to-all writes them at the
- * arena's end): d_rec_off holds arena word offsets, the key of the first record of a sequence becomes the table's
- * copy, nothing is moved.  The caller advances the arena counter (d_ctrl[0]) past the received words. */
+/* Merge (key, count) records received straight into the table's arena (the all-to-all writes them at the arena's
+ * end): record i = [count][key words...] at arena word offset d_rec_off[i].  The key of the first record of a
+ * sequence becomes the table's copy, nothing is moved.  Used by the owner side of the hash-partitioned exchange; the
+ * caller advances the arena counter (d_ctrl[0]) past the received words. */
 int mirge_collapse_merge_inplace(mirge_ctx *ctx, const mirge_table *t, const uint32_t *d_rec_off, uint64_t n_rec,
                                  uint32_t *d_deferred, void *stream);
 /* Growth: re-insert every slot of old_t into the larger slot array of new_t (zeroed here).  Both
@@ -329,13 +305,8 @@ int mirge_pack_keys(mirge_ctx *ctx, const uint8_t *d_ascii, const uint64_t *d_st
 int mirge_partition_plan(mirge_ctx *ctx, const mirge_table *t, const uint32_t *d_ids, uint64_t n,
                          int umi5, int umi3, uint32_t n_parts, uint32_t *d_dest, uint32_t *d_words,
                          void *stream);
-/* Write exchange records [count][key words] of pairs (d_ids[i], d_counts[i]) at word offsets
- * d_rec_off[i] of d_rec. */
-int mirge_partition_pack(mirge_ctx *ctx, const mirge_table *t, const uint32_t *d_ids,
-                         const uint32_t *d_counts, uint64_t n, const uint32_t *d_rec_off,
-                         uint32_t *d_rec, void *stream);
-
-/* The same packing without sorting by destination.  mirge_partition_totals: d_totals[d] = words and
+/* Exchange records [count][key words] of pairs (d_ids[i], d_counts[i]), grouped by destination without a sort.
+ * mirge_partition_totals: d_totals[d] = words and
  * d_totals[n_parts + d] = records bound for destination d (u64[2 * n_parts], zeroed here; n_parts <= 64).
  * mirge_partition_scatter: d_cursors (u64[n_parts]) holds, per destination, (first record index of its region in
  * d_sizes) << 32 | (first word offset of its region in d_rec), both < 2^32; every pair is written as [count][key words] at the offset
@@ -348,7 +319,7 @@ int mirge_partition_scatter(mirge_ctx *ctx, const mirge_table *t, const uint32_t
 
 /* Sharding BEFORE the collapse (reads of one sample spread over the ranks; the reference's counterpart is the
  * parent loop that merges the workers' dictionaries, digest.py:141-163): the insert list of a batch (d_keys, d_ins as
- * mirge_trim / mirge_digest_tiles wrote them) is cut by owner = hash(key) mod n_parts into n_parts regions of
+ * mirge_trim wrote them) is cut by owner = hash(key) mod n_parts into n_parts regions of
  * d_out_items (u64 = {u32 word offset of the key inside the region's keys, u32 count}; region d starts at d * cap_items)
  * and d_out_keys (region d starts at word d * cap_words).  d_cursors[d] (u64[n_parts], zeroed here) = items << 32 | key
  * words bound for d -- it keeps counting when a region is full; the caller then repeats with regions that large.

@@ -113,7 +113,7 @@ class RoundPolicy(C.Structure):
     ]
 
 
-ABI_VERSION = 3  # MIRGE_ABI_VERSION of include/mirge_b200.h
+ABI_VERSION = 4  # MIRGE_ABI_VERSION of include/mirge_b200.h
 
 # name -> (restype, argtypes); every symbol include/mirge_b200.h declares
 _P = C.c_void_p
@@ -132,12 +132,8 @@ SYMBOLS = {
     "mirge_trim_scratch_bytes": (_U64, [_U64]),
     "mirge_trim": (C.c_int, [_P, _P, _U64, _P, _U64, _P, _P, _P, _U64, _P, _P, _P, _U64, _P]),
     "mirge_trim_mode": (C.c_int, [_P, C.c_int]),
-    "mirge_digest_fused_ok": (C.c_int, [_P]),
-    "mirge_digest_scratch_bytes": (_U64, [_U64, _U64]),
-    "mirge_digest_tiles": (C.c_int, [_P, _P, _U64, C.c_int, _U64, _P, _P, _P, _P, _U64, _P, _P, _P, _U64, _P]),
     "mirge_table_reset": (C.c_int, [_P, C.POINTER(Table), _P]),
     "mirge_collapse_insert_list": (C.c_int, [_P, C.POINTER(Table), _P, _P, _U64, _P, _P]),
-    "mirge_collapse_merge": (C.c_int, [_P, C.POINTER(Table), _P, _P, _U64, _P, _P]),
     "mirge_collapse_merge_inplace": (C.c_int, [_P, C.POINTER(Table), _P, _U64, _P, _P]),
     "mirge_table_rehash": (C.c_int, [_P, C.POINTER(Table), C.POINTER(Table), _P]),
     "mirge_table_check_sync":(C.c_int, [_P, C.POINTER(Table), _PU64, _PU64, _P]),
@@ -153,7 +149,6 @@ SYMBOLS = {
         C.c_int,
         [_P, C.POINTER(Table), _P, _U64, C.c_int, C.c_int, C.c_uint32, _P, _P, _P],
     ),
-    "mirge_partition_pack": (C.c_int, [_P, C.POINTER(Table), _P, _P, _U64, _P, _P, _P]),
     "mirge_partition_totals": (C.c_int, [_P, _P, _P, _U64, C.c_uint32, _P, _P]),
     "mirge_partition_scatter": (C.c_int, [_P, C.POINTER(Table), _P, _P, _P, _P, _U64, C.c_uint32, _P, _P, _P, _P]),
     "mirge_shard_scatter": (C.c_int, [_P, _P, _P, _U64, C.c_uint32, C.c_uint32, C.c_uint32, _P, _P, _P, _P]),

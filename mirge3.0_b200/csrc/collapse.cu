@@ -158,17 +158,15 @@ __device__ __forceinline__ void defer_item(unsigned long long *counter, uint32_t
   list[base + __popc(grp & ((1u << lane) - 1u))] = item;
 }
 
-// Exchange records of the owner-side merge.  mode 1: records [count][key...] at rec_off[i] of `keys`;
-// mode 3: records that were received straight into the table's arena (keys == arena): the key of a record becomes
-// the table's copy where it lies, nothing is moved.
-__device__ __forceinline__ void item_key(int mode, const uint32_t *keys, const uint32_t *off, uint64_t i,
+// Exchange records of the owner-side merge: records [count][key...] at rec_off[i] that were received straight into
+// the table's arena (keys == arena): the key of a record becomes the table's copy where it lies, nothing is moved.
+__device__ __forceinline__ void item_key(const uint32_t *keys, const uint32_t *off, uint64_t i,
                                          const uint32_t *&key, uint32_t &add, uint32_t &in_arena) {
   const uint32_t o = off[i];
-  in_arena = NOT_IN_ARENA;
-  if (o == 0xFFFFFFFFu) { key = nullptr; add = 0; return; }
+  if (o == 0xFFFFFFFFu) { key = nullptr; add = 0; in_arena = NOT_IN_ARENA; return; }
   key = keys + o + 1;
   add = keys[o];
-  if (mode == 3) in_arena = o + 1;
+  in_arena = o + 1;
 }
 
 // Hash of an in-arena key whose length is not known yet: the header and the next seven words are fetched together
@@ -188,28 +186,21 @@ __device__ __forceinline__ uint64_t hash_key_in_arena(const mirge_table &t, cons
 
 __global__ void __launch_bounds__(COL_THREADS)
 collapse_insert_kernel(mirge_table t, const uint32_t *__restrict__ keys, const uint32_t *__restrict__ off, uint64_t n,
-                       int mode, uint32_t *__restrict__ deferred) {
+                       uint32_t *__restrict__ deferred) {
   const uint64_t i = (uint64_t)blockIdx.x * COL_THREADS + threadIdx.x;
   if (i >= n) return;
   const uint32_t *key; uint32_t add, in_arena;
-  item_key(mode, keys, off, i, key, add, in_arena);
+  item_key(keys, off, i, key, add, in_arena);
   if (!key || add == 0) return;
-  uint32_t nw;
-  uint64_t h;
-  if (mode == 3) {  // uniform: the keys lie in the table's arena
-    uint32_t kw[8];
-    h = hash_key_in_arena(t, key, in_arena, nw, kw);
-  } else {
-    nw = key_words(key[0]);
-    h = hash_key(key, nw);
-  }
+  uint32_t nw, kw[8];
+  const uint64_t h = hash_key_in_arena(t, key, in_arena, nw, kw);
   if (table_insert<false>(t, key, nw, add, h, false, in_arena) == INS_DEFER)
     defer_item((unsigned long long *)t.d_ctrl + 3, deferred, (uint32_t)i);
 }
 
 // drains the deferred list: one lane per warp, so a waiter never shares a warp with its claimant
 __global__ void __launch_bounds__(COL_THREADS)
-collapse_retry_kernel(mirge_table t, const uint32_t *__restrict__ keys, const uint32_t *__restrict__ off, uint64_t n, int mode,
+collapse_retry_kernel(mirge_table t, const uint32_t *__restrict__ keys, const uint32_t *__restrict__ off, uint64_t n,
                       const uint32_t *__restrict__ deferred) {
   if (threadIdx.x & 31) return;
   const unsigned long long nd = ((unsigned long long *)t.d_ctrl)[3];
@@ -218,7 +209,7 @@ collapse_retry_kernel(mirge_table t, const uint32_t *__restrict__ keys, const ui
   for (uint64_t j = warp; j < nd; j += nwarps) {
     const uint64_t i = deferred[j];
     const uint32_t *key; uint32_t add, in_arena;
-    item_key(mode, keys, off, i, key, add, in_arena);
+    item_key(keys, off, i, key, add, in_arena);
     if (!key) continue;
     const uint32_t nw = key_words(key[0]);
     table_insert<false>(t, key, nw, add, hash_key(key, nw), true, in_arena);
@@ -385,24 +376,6 @@ extern "C" int mirge_table_reset(mirge_ctx *ctx, const mirge_table *t, void *str
   return MIRGE_OK;
 }
 
-static int run_insert(mirge_ctx *ctx, const mirge_table *t, const uint32_t *keys, const uint32_t *off, uint64_t n, int mode,
-                      uint32_t *d_deferred, cudaStream_t stream) {
-  int rc = check_table(ctx, t);
-  if (rc) return rc;
-  if (n == 0) return MIRGE_OK;
-  if (!keys || !off || !d_deferred) MIRGE_FAIL(ctx, MIRGE_ERR_ARG, "collapse: null buffer");
-  if (n > 0xFFFFFFFFull) MIRGE_FAIL(ctx, MIRGE_ERR_ARG, "collapse: more than 2^32 items in one batch");
-  MIRGE_CUDA(ctx, cudaSetDevice(ctx->device));
-  const unsigned grid = (unsigned)((n + COL_THREADS - 1) / COL_THREADS);
-  collapse_insert_kernel<<<grid, COL_THREADS, 0, stream>>>(*t, keys, off, n, mode, d_deferred);
-  MIRGE_LAUNCH_CHECK(ctx, "collapse_insert_kernel");
-  collapse_retry_kernel<<<ctx->sm_count, COL_THREADS, 0, stream>>>(*t, keys, off, n, mode, d_deferred);
-  MIRGE_LAUNCH_CHECK(ctx, "collapse_retry_kernel");
-  clear_deferred_kernel<<<1, 1, 0, stream>>>((unsigned long long *)t->d_ctrl);
-  MIRGE_LAUNCH_CHECK(ctx, "clear_deferred_kernel");
-  return MIRGE_OK;
-}
-
 extern "C" int mirge_collapse_insert_list(mirge_ctx *ctx, const mirge_table *t, const uint32_t *d_keys, const uint64_t *d_ins,
                                           uint64_t n_items, uint32_t *d_scratch, void *stream_) {
   if (!ctx) return MIRGE_ERR_ARG;
@@ -439,17 +412,25 @@ extern "C" int mirge_collapse_insert_list(mirge_ctx *ctx, const mirge_table *t, 
   return MIRGE_OK;
 }
 
-extern "C" int mirge_collapse_merge(mirge_ctx *ctx, const mirge_table *t, const uint32_t *d_rec, const uint32_t *d_rec_off,
-                                    uint64_t n_rec, uint32_t *d_deferred, void *stream) {
-  if (!ctx) return MIRGE_ERR_ARG;
-  return run_insert(ctx, t, d_rec, d_rec_off, n_rec, 1, d_deferred, (cudaStream_t)stream);
-}
-
 extern "C" int mirge_collapse_merge_inplace(mirge_ctx *ctx, const mirge_table *t, const uint32_t *d_rec_off, uint64_t n_rec,
-                                            uint32_t *d_deferred, void *stream) {
+                                            uint32_t *d_deferred, void *stream_) {
   if (!ctx) return MIRGE_ERR_ARG;
   if (!t) MIRGE_FAIL(ctx, MIRGE_ERR_ARG, "collapse: null table");
-  return run_insert(ctx, t, t->d_arena, d_rec_off, n_rec, 3, d_deferred, (cudaStream_t)stream);
+  int rc = check_table(ctx, t);
+  if (rc) return rc;
+  if (n_rec == 0) return MIRGE_OK;
+  if (!d_rec_off || !d_deferred) MIRGE_FAIL(ctx, MIRGE_ERR_ARG, "collapse: null buffer");
+  if (n_rec > 0xFFFFFFFFull) MIRGE_FAIL(ctx, MIRGE_ERR_ARG, "collapse: more than 2^32 items in one batch");
+  cudaStream_t stream = (cudaStream_t)stream_;
+  MIRGE_CUDA(ctx, cudaSetDevice(ctx->device));
+  const unsigned grid = (unsigned)((n_rec + COL_THREADS - 1) / COL_THREADS);
+  collapse_insert_kernel<<<grid, COL_THREADS, 0, stream>>>(*t, t->d_arena, d_rec_off, n_rec, d_deferred);
+  MIRGE_LAUNCH_CHECK(ctx, "collapse_insert_kernel");
+  collapse_retry_kernel<<<ctx->sm_count, COL_THREADS, 0, stream>>>(*t, t->d_arena, d_rec_off, n_rec, d_deferred);
+  MIRGE_LAUNCH_CHECK(ctx, "collapse_retry_kernel");
+  clear_deferred_kernel<<<1, 1, 0, stream>>>((unsigned long long *)t->d_ctrl);
+  MIRGE_LAUNCH_CHECK(ctx, "clear_deferred_kernel");
+  return MIRGE_OK;
 }
 
 extern "C" int mirge_table_check_sync(mirge_ctx *ctx, const mirge_table *t, uint64_t *n_keys, uint64_t *arena_used, void *stream_) {
@@ -752,32 +733,6 @@ extern "C" int mirge_partition_plan(mirge_ctx *ctx, const mirge_table *t, const 
   MIRGE_CUDA(ctx, cudaSetDevice(ctx->device));
   partition_plan_kernel<<<(unsigned)((n + 127) / 128), 128, 0, stream>>>(*t, d_ids, n, umi5, umi3, n_parts, d_dest, d_words);
   MIRGE_LAUNCH_CHECK(ctx, "partition_plan_kernel");
-  return MIRGE_OK;
-}
-
-__global__ void __launch_bounds__(COL_THREADS)
-partition_pack_kernel(mirge_table t, const uint32_t *__restrict__ ids, const uint32_t *__restrict__ counts, uint64_t n,
-                      const uint32_t *__restrict__ rec_off, uint32_t *__restrict__ rec) {
-  const uint64_t i = (uint64_t)blockIdx.x * COL_THREADS + threadIdx.x;
-  if (i >= n) return;
-  const uint32_t *key = t.d_arena + t.d_key_ref[ids[i]];
-  const uint32_t nw = key_words(key[0]);
-  uint32_t *o = rec + rec_off[i];
-  o[0] = counts[i];
-  for (uint32_t w = 0; w < nw; ++w) o[1 + w] = key[w];
-}
-
-extern "C" int mirge_partition_pack(mirge_ctx *ctx, const mirge_table *t, const uint32_t *d_ids, const uint32_t *d_counts, uint64_t n,
-                                    const uint32_t *d_rec_off, uint32_t *d_rec, void *stream_) {
-  if (!ctx) return MIRGE_ERR_ARG;
-  int rc = check_table(ctx, t);
-  if (rc) return rc;
-  if (n == 0) return MIRGE_OK;
-  if (!d_ids || !d_counts || !d_rec_off || !d_rec) MIRGE_FAIL(ctx, MIRGE_ERR_ARG, "partition_pack: null buffer");
-  cudaStream_t stream = (cudaStream_t)stream_;
-  MIRGE_CUDA(ctx, cudaSetDevice(ctx->device));
-  partition_pack_kernel<<<(unsigned)((n + COL_THREADS - 1) / COL_THREADS), COL_THREADS, 0, stream>>>(*t, d_ids, d_counts, n, d_rec_off, d_rec);
-  MIRGE_LAUNCH_CHECK(ctx, "partition_pack_kernel");
   return MIRGE_OK;
 }
 

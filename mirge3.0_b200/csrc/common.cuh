@@ -118,36 +118,3 @@ __device__ __forceinline__ uint32_t newline_mask(const uint32_t w[8]) {
   }
   return m;
 }
-
-// ---------------------------------------------------------------- mbarrier / bulk copy (TMA) ----
-// Shared-memory barriers with transaction counts and the 1-D bulk copy engine (cp.async.bulk): one elected thread
-// arms the barrier with the byte count and issues the copy; waiters poll the phase parity.
-__device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint64_t *bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t *bar) {
-  asm volatile("{\n\t.reg .b64 st;\n\tmbarrier.arrive.shared::cta.b64 st, [%0];\n\t}" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive_expect_tx(uint64_t *bar, uint32_t bytes) {
-  asm volatile("{\n\t.reg .b64 st;\n\tmbarrier.arrive.expect_tx.shared::cta.b64 st, [%0], %1;\n\t}" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ bool mbar_try_wait(uint64_t *bar, uint32_t parity) {
-  uint32_t ok;
-  asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-               : "=r"(ok) : "r"(smem_u32(bar)), "r"(parity) : "memory");
-  return ok != 0;
-}
-#ifndef MBAR_SLEEP
-#define MBAR_SLEEP 0
-#endif
-__device__ __forceinline__ void mbar_wait(uint64_t *bar, uint32_t parity) {
-  while (!mbar_try_wait(bar, parity)) {
-    if (MBAR_SLEEP) __nanosleep(MBAR_SLEEP);  // a waiting warp leaves the issue slots to the warps that work
-  }
-}
-// global -> shared bulk copy of `bytes` (multiple of 16; both addresses 16-byte aligned), completion counted on `bar`
-__device__ __forceinline__ void bulk_load(void *smem_dst, const void *gmem_src, uint32_t bytes, uint64_t *bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(smem_u32(smem_dst)),
-               "l"(gmem_src), "r"(bytes), "r"(smem_u32(bar)) : "memory");
-}

@@ -115,19 +115,6 @@ struct DpEntry {
   uint32_t pad;
 };
 
-// A record the fused tokenise + stage-1 kernel leaves to the whole-pipeline pass: it has no line index to point
-// into, so the entry carries the record's line starts (offsets in the aligned stream).  y == 0: only the header
-// start x is known (the record reaches beyond the tile's overhang); the pass finds the line breaks itself.
-struct SlowRec {
-  uint32_t r, x, y, z, w, nxt, pad0, pad1;
-};
-// where deferred records go: record indices (a line index exists) or full entries
-struct SlowSink {
-  uint32_t *r_list;
-  SlowRec *recs;
-  uint64_t cap;  // entries of recs (r_list holds one per record of the batch)
-};
-
 // first adapter modifier, and the number of emission slots stage 1 owns for a read that goes on to the search
 __device__ __forceinline__ int first_adapter_mod() {
   int mi_ad = c_p.n_mods;
@@ -198,14 +185,14 @@ __device__ __forceinline__ void flush_stats(unsigned long long *ctrl) {
 // Sizes, key space (one atomic per warp), second-pass queue and the writes of emission slots [slot_lo, slot_hi)
 // of record r.  All 32 lanes of a warp must call it together.  fast_emit: the keys are slices of the packed
 // pure-ACGT read in ps_mine; otherwise they are packed from the bytes in seq (exceptions included).
-// to_slow: PASS 1 only, queues the record for the second pass (which redoes it from scratch).
+// to_slow: PASS 1 only, queues the record index in d_slow for the second pass (which redoes it from scratch).
 template <bool FAST, int PASS>
 __device__ __forceinline__ void emit_record(const bool valid, const uint64_t r, const int E, const int slot_lo, const int slot_hi,
                                             const uint8_t *seq, const bool fast_emit, const int *w_start, const int *w_stop,
                                             const int *w_us, const int *w_ue, uint32_t *w_words, const bool to_slow,
                                             ushort4 *__restrict__ win, uint32_t *__restrict__ key_off, uint32_t *__restrict__ keys,
-                                            uint64_t keys_cap, unsigned long long *__restrict__ ctrl, const SlowSink ss, const uint4 ls,
-                                            const uint32_t nxt, const uint32_t *ps_mine, const InsList il) {
+                                            uint64_t keys_cap, unsigned long long *__restrict__ ctrl, uint32_t *__restrict__ d_slow,
+                                            const uint32_t *ps_mine, const InsList il) {
   const int lane = threadIdx.x & 31;
   uint32_t my_words = 0, my_kept = 0, my_alg = 0, same_as_prev = 0, my_items = 0;
   if (valid) {
@@ -270,19 +257,7 @@ __device__ __forceinline__ void emit_record(const bool valid, const uint64_t r, 
       unsigned long long base = 0;
       if (lane == __ffs(sm_) - 1) base = atomicAdd(ctrl + 5, (unsigned long long)__popc(sm_));
       base = __shfl_sync(0xffffffffu, base, __ffs(sm_) - 1);
-      if (to_slow) {
-        const unsigned long long at = base + __popc(sm_ & ((1u << lane) - 1u));
-        if (!ss.recs) {
-          ss.r_list[at] = (uint32_t)r;
-        } else if (at < ss.cap) {
-          SlowRec sr;
-          sr.r = (uint32_t)r; sr.x = ls.x; sr.y = ls.y; sr.z = ls.z; sr.w = ls.w; sr.nxt = nxt; sr.pad0 = sr.pad1 = 0;
-          *(uint4 *)&ss.recs[at] = *(const uint4 *)&sr;
-          *((uint4 *)&ss.recs[at] + 1) = *((const uint4 *)&sr + 1);
-        } else {
-          atomicOr(ctrl + 2, 8ull);  // list full: the host repeats the batch on the two-pass path
-        }
-      }
+      if (to_slow) d_slow[base + __popc(sm_ & ((1u << lane) - 1u))] = (uint32_t)r;
     }
   }
   if (!valid) return;
@@ -364,7 +339,7 @@ template <int MAXM, bool FAST, int PASS, bool SPLIT>
 __device__ __forceinline__ void process_record(const bool valid, const uint64_t r, const uint8_t *B, uint64_t nbytes,
                                                const uint32_t *__restrict__ line_start, ushort4 *__restrict__ win,
                                                uint32_t *__restrict__ key_off, uint32_t *__restrict__ keys, uint64_t keys_cap,
-                                               unsigned long long *__restrict__ ctrl, const SlowSink ss, FastCtx &fc,
+                                               unsigned long long *__restrict__ ctrl, uint32_t *__restrict__ d_slow, FastCtx &fc,
                                                uint32_t *ps_mine, const SplitOut so, const uint4 ls, const uint32_t nxt,
                                                const InsList il) {
   const int lane = threadIdx.x & 31;
@@ -544,22 +519,7 @@ __device__ __forceinline__ void process_record(const bool valid, const uint64_t 
     }
   }
   emit_record<FAST, PASS>(valid, r, E, slot_lo, slot_hi, seq, fast_emit, w_start, w_stop, w_us, w_ue, w_words, to_slow, win, key_off,
-                          keys, keys_cap, ctrl, ss, ls, nxt, ps_mine, il);
-}
-
-// Line starts of the record whose header begins at ls.x, found in the global stream (records the fused kernel
-// could not see whole).  virtual_nl: the stream is the end of the input and its last line has no line break.
-// false: the stream ends before the record is complete (it belongs to the next batch, or the file is truncated).
-__device__ __noinline__ bool find_lines(const uint8_t *fq, uint64_t n, uint4 &ls, uint32_t &nxt, bool virtual_nl) {
-  uint32_t found[4];
-  int k = 0;
-  for (uint64_t p = ls.x; p < n && k < 4; ++p)
-    if (fq[p] == '\n') found[k++] = (uint32_t)p + 1u;
-  if (k == 3 && virtual_nl && n > found[2]) found[k++] = (uint32_t)n + 1u;
-  if (k < 4) return false;
-  ls.y = found[0]; ls.z = found[1]; ls.w = found[2];
-  nxt = found[3];
-  return true;
+                          keys, keys_cap, ctrl, d_slow, ps_mine, il);
 }
 
 // FAST = bit-parallel adapter search (locate_fast) + packed-read key emission; requires the CTA's span to be
@@ -570,7 +530,7 @@ __global__ void __launch_bounds__(TRIM_THREADS, (FAST && PASS == 1) ? 7 : 1)
 trim_kernel(const uint8_t *__restrict__ fq, uint64_t nbytes, const uint32_t *__restrict__ line_start, uint64_t n_records,
             ushort4 *__restrict__ win, uint32_t *__restrict__ key_off, uint32_t *__restrict__ keys, uint64_t keys_cap,
             unsigned long long *__restrict__ ctrl, uint32_t smem_bytes, uint32_t *__restrict__ d_slow, const SplitOut so,
-            const InsList il, const int pack_words, const SlowRec *__restrict__ slow_recs, const uint32_t n_cap) {
+            const InsList il, const int pack_words) {
   extern __shared__ uint4 smem4[];
   uint8_t *sbuf = (uint8_t *)smem4;
   const int tid = threadIdx.x;
@@ -589,41 +549,25 @@ trim_kernel(const uint8_t *__restrict__ fq, uint64_t nbytes, const uint32_t *__r
     ps_mine = eq + c_p.n_adapters * 256 + tid;
     fc.ps = ps_mine;
   }
-  const SlowSink ss{d_slow, nullptr, 0};
   if (PASS == 2) {
     // second pass: the deferred reads, addressed in the global stream; whole warps iterate together
     __syncthreads();
-    unsigned long long n_slow = ctrl[5];
-    if (slow_recs && n_slow > n_cap) n_slow = n_cap;  // (entries beyond the list were not written; the batch is flagged)
+    const unsigned long long n_slow = ctrl[5];
     const uint64_t first = (uint64_t)blockIdx.x * TRIM_THREADS + (tid & ~31);
     for (uint64_t base = first; base < n_slow; base += (uint64_t)gridDim.x * TRIM_THREADS) {
       const uint64_t idx = base + (tid & 31);
-      bool valid = idx < n_slow;
+      const bool valid = idx < n_slow;
       uint64_t r = 0;
       fc.jump_ok = false;
       uint4 ls = make_uint4(0, 0, 0, 0);
       uint32_t nxt = 0;
-      if (valid && slow_recs) {  // entries of the fused kernel: the line starts travel with the record
-        const uint4 a = *(const uint4 *)&slow_recs[idx], b = *((const uint4 *)&slow_recs[idx] + 1);
-        r = a.x;
-        ls = make_uint4(a.y, a.z, a.w, b.x);
-        nxt = b.y;
-        if (ls.y == 0) valid = find_lines(fq, nbytes, ls, nxt, b.z != 0);  // a record beyond its tile's overhang
-        if (valid && r >= n_cap) {
-          atomicOr(ctrl + 2, 16ull);
-          valid = false;
-        }
-        if (valid && line_start) {
-          uint32_t *lo = const_cast<uint32_t *>(line_start);
-          lo[4 * r] = ls.x; lo[4 * r + 1] = ls.y; lo[4 * r + 2] = ls.z; lo[4 * r + 3] = ls.w; lo[4 * r + 4] = nxt;
-        }
-      } else if (valid) {
+      if (valid) {
         r = d_slow[idx];
         ls = *(const uint4 *)(line_start + 4 * r);
         nxt = line_start[4 * r + 4];
       }
       process_record<MAXM, FAST, 2, false>(valid, r, fq, nbytes, line_start, win, key_off, keys, keys_cap, ctrl,
-                                           ss, fc, ps_mine, so, ls, nxt, il);
+                                           d_slow, fc, ps_mine, so, ls, nxt, il);
       __syncwarp();
     }
     flush_stats(ctrl);
@@ -670,327 +614,7 @@ trim_kernel(const uint8_t *__restrict__ fq, uint64_t nbytes, const uint32_t *__r
   uint32_t nxt = 0;
   if (valid) { ls = *(const uint4 *)(line_start + 4 * r); nxt = line_start[4 * r + 4]; }
   const uint8_t *B = staged ? (const uint8_t *)(sbuf - alo) : fq;  // B[absolute stream offset]
-  process_record<MAXM, FAST, PASS, SPLIT>(valid, r, B, nbytes, line_start, win, key_off, keys, keys_cap, ctrl, ss, fc, ps_mine, so, ls, nxt, il);
-  flush_stats(ctrl);
-}
-
-// ---- fused tokeniser + stage 1: persistent, warp-specialised, fed by the bulk-copy engine ---------------------------
-// The two-pass path streams the FASTQ bytes twice (newline census + line index, then the staging of stage 1) and
-// stages with per-thread copies.  Here a persistent CTA (one producer warp, DT_GROUPS x 4 consumer warps) walks the
-// stream in tiles of DT_TILE bytes handed out by a global ticket:
-//   producer: one elected lane arms an mbarrier with the tile's byte count and issues ONE bulk copy (cp.async.bulk,
-//     the 1-D TMA path) of tile + overhang into a shared-memory buffer; while the consumers work on the previous
-//     buffer it scans the new one for line breaks (32 bytes per lane and step, same arithmetic as the census kernel)
-//     into a bit mask + running counts in shared memory, learns the number of line breaks before its tile from the
-//     tiles in front of it (decoupled look-back over per-tile aggregates, single pass), and publishes the tile:
-//     which line breaks start a record (every fourth, by the global count), how many records, the index of the first.
-//   consumers: take 32 records at a time from the published tile (shared-memory ticket), find their five line
-//     breaks in the mask (one binary search over the running counts, then bit scans), and run stage 1 of the split
-//     pipeline on the bytes in shared memory -- the same process_record as the two-pass path.
-// A tile owns the records whose preceding line break lies in it; a record that reaches beyond the overhang (or
-// that stage 1 hands on anyway: non-ACGT characters, long reads) goes to the whole-pipeline pass with its line
-// starts.  Buffers cycle through full (bulk copy done) -> ready (scanned) -> empty (all consumer warps done)
-// mbarriers; nothing in the loop is a CTA-wide barrier.
-#ifndef DT_TILE
-#define DT_TILE 16384
-#endif
-#define DT_OVH 2048
-#define DT_LOAD (DT_TILE + DT_OVH)
-#define DT_WORDS (DT_LOAD / 32)
-#ifndef DT_NBUF
-#define DT_NBUF 2
-#endif
-#ifndef DT_GROUPS
-#define DT_GROUPS 1
-#endif
-#define DT_CWARPS (DT_GROUPS * TRIM_THREADS / 32)
-#define DT_THREADS (32 + DT_GROUPS * TRIM_THREADS)
-#define DT_FLAG_AGG (1ull << 62)
-#define DT_FLAG_INC (2ull << 62)
-#define DT_VAL_MASK ((1ull << 62) - 1ull)
-static_assert(DT_TILE % 1024 == 0 && DT_LOAD % 1024 == 0, "the producer scans 1 KB per step");
-
-struct TileMeta {
-  unsigned long long before;   // line breaks of the stream in front of the tile
-  unsigned long long tile_lo;  // stream offset of the tile
-  uint32_t n_rec;              // records the tile owns (0xFFFFFFFF: no more tiles)
-  uint32_t j0;                 // ordinal (in the loaded range) of the line break in front of its first record
-  uint32_t nload;              // bytes of the loaded range
-  uint32_t first;              // 1: the tile also owns record 0 of the stream (no line break in front of it)
-  uint32_t n_nl;               // line breaks in the loaded range
-  uint32_t at_end;             // the loaded range reaches the end of the stream
-};
-
-struct DigestTilesArgs {
-  const uint8_t *fq;           // 16-byte aligned stream
-  unsigned long long n;        // its bytes
-  uint32_t skew;               // first byte that belongs to the batch
-  uint32_t is_final;
-  unsigned long long n_tiles;
-  unsigned long long *tile_state;
-  uint32_t *line_start;        // optional output (parity tests)
-  uint32_t n_cap;              // records the per-record outputs / lists have room for
-  ushort4 *win;
-  uint32_t *key_off;
-  uint32_t *keys;
-  unsigned long long keys_cap;
-  unsigned long long *ctrl;
-  SlowSink ss;
-  SplitOut so;
-  InsList il;
-  int pack_words;
-};
-
-// position (in the loaded range) of line break number j of the range: binary search over the running counts of the
-// 32-byte pieces, then the bit inside the piece
-__device__ __forceinline__ uint32_t nl_position(const uint32_t *mask, const uint16_t *pref, uint32_t j, uint32_t &w_out) {
-  uint32_t lo = 0, hi = DT_WORDS;  // largest w with pref[w] <= j
-  while (hi - lo > 1) {
-    const uint32_t mid = (lo + hi) >> 1;
-    if (pref[mid] <= j) lo = mid; else hi = mid;
-  }
-  uint32_t m = mask[lo];
-  for (uint32_t k = j - pref[lo]; k; --k) m &= m - 1;
-  w_out = lo;
-  return 32u * lo + (uint32_t)(__ffs((int)m) - 1);
-}
-// the next line break after position p (piece w); 0xFFFFFFFF when the loaded range has none
-__device__ __forceinline__ uint32_t nl_next(const uint32_t *mask, uint32_t p, uint32_t &w) {
-  const uint32_t bit = p & 31u;
-  uint32_t m = bit == 31u ? 0u : (mask[w] & (0xFFFFFFFEu << bit));
-  while (m == 0u) {
-    if (++w >= DT_WORDS) return 0xFFFFFFFFu;
-    m = mask[w];
-  }
-  return 32u * w + (uint32_t)(__ffs((int)m) - 1);
-}
-
-__global__ void __launch_bounds__(DT_THREADS, 3) digest_tiles_kernel(const __grid_constant__ DigestTilesArgs A) {
-  extern __shared__ uint4 smem4[];
-  __shared__ uint64_t bar_full[DT_NBUF], bar_ready[DT_NBUF], bar_empty[DT_NBUF];
-  __shared__ TileMeta s_meta[DT_NBUF];
-  __shared__ uint32_t s_next[DT_NBUF];
-  // smem: [buffers DT_NBUF x DT_LOAD][masks DT_NBUF x DT_WORDS][counts DT_NBUF x (DT_WORDS + 2) u16][eq tables][packed rows]
-  uint8_t *bufs = (uint8_t *)smem4;
-  uint32_t *masks = (uint32_t *)(bufs + DT_NBUF * DT_LOAD);
-  uint16_t *prefs = (uint16_t *)(masks + DT_NBUF * DT_WORDS);
-  uint32_t *eq = (uint32_t *)(prefs + DT_NBUF * (DT_WORDS + 2));
-  uint32_t *ps_base = eq + c_p.n_adapters * 256;
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  unsigned long long *ctrl = A.ctrl;
-  init_stats(A.pack_words);
-  for (int e = tid; e < c_p.n_adapters * 256; e += DT_THREADS) {
-    const uint32_t code = base_code_upper((uint32_t)(e & 255));
-    eq[e] = code < 4u ? (uint32_t)c_p.ad[e >> 8].peq[code] : 0u;
-  }
-  if (tid == 0) {
-    for (int b = 0; b < DT_NBUF; ++b) {
-      mbar_init(&bar_full[b], 1);
-      mbar_init(&bar_ready[b], 1);
-      mbar_init(&bar_empty[b], DT_CWARPS);
-    }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  __syncthreads();
-  const bool virtual_nl = A.is_final && A.n > A.skew && A.fq[A.n - 1] != '\n';  // EOF rule: the last line is complete without '\n'
-
-  if (warp == 0) {
-    // ------------------------------------------------------------------ producer
-    for (uint32_t it = 0;; ++it) {
-      const int b = it % DT_NBUF;
-      const uint32_t par = (it / DT_NBUF) & 1u;
-      if (it >= DT_NBUF) mbar_wait(&bar_empty[b], par ^ 1u);  // the consumers are done with this buffer's previous tile
-      unsigned long long t = 0;
-      if (lane == 0) t = atomicAdd(ctrl + 11, 1ull);
-      t = __shfl_sync(0xffffffffu, t, 0);
-      TileMeta &M = s_meta[b];
-      if (t >= A.n_tiles) {
-        if (lane == 0) {
-          M.n_rec = 0xFFFFFFFFu;
-          mbar_arrive(&bar_ready[b]);
-        }
-        break;
-      }
-      const unsigned long long tile_lo = t * DT_TILE;
-      const uint32_t nload = (uint32_t)min((unsigned long long)DT_LOAD, A.n - tile_lo);
-      const uint32_t bulk = nload & ~15u;
-      uint8_t *buf = bufs + b * DT_LOAD;
-      if (lane == 0) {
-        if (bulk) {
-          mbar_arrive_expect_tx(&bar_full[b], bulk);
-          bulk_load(buf, A.fq + tile_lo, bulk, &bar_full[b]);
-        } else {
-          mbar_arrive(&bar_full[b]);
-        }
-      }
-      if ((uint32_t)lane < nload - bulk) buf[bulk + lane] = A.fq[tile_lo + bulk + lane];  // the last bytes of the stream
-      __syncwarp();
-      mbar_wait(&bar_full[b], par);
-      // line breaks of the loaded range: bit mask per 32 bytes + running count in front of every piece
-      uint32_t *mk = masks + b * DT_WORDS;
-      uint16_t *pf = prefs + b * (DT_WORDS + 2);
-      const uint32_t vpos = (virtual_nl && A.n - tile_lo < DT_LOAD) ? (uint32_t)(A.n - tile_lo) : 0xFFFFFFFFu;
-      uint32_t running = 0, tile_total = 0;
-#pragma unroll 1
-      for (uint32_t w0 = 0; w0 < DT_WORDS; w0 += 32) {
-        const uint32_t w = w0 + lane, pos = 32u * w;
-        uint32_t m = 0;
-        if (pos < nload) {
-          const uint4 a = *(const uint4 *)(buf + pos), c = *(const uint4 *)(buf + pos + 16);
-          const uint32_t ww[8] = {a.x, a.y, a.z, a.w, c.x, c.y, c.z, c.w};
-          m = newline_mask(ww);
-          if (pos + 32 > nload) m &= (1u << (nload - pos)) - 1u;  // bytes behind the stream's end are not ours
-          if (t == 0 && w == 0) m &= ~((1u << A.skew) - 1u);     // nor the ones in front of the batch
-        }
-        if (vpos >= pos && vpos < pos + 32) m |= 1u << (vpos - pos);
-        mk[w] = m;
-        const uint32_t c = __popc(m);
-        uint32_t inc = c;
-#pragma unroll
-        for (int d = 1; d < 32; d <<= 1) {
-          const uint32_t x = __shfl_up_sync(0xffffffffu, inc, d);
-          if (lane >= d) inc += x;
-        }
-        pf[w] = (uint16_t)(running + inc - c);
-        running += __shfl_sync(0xffffffffu, inc, 31);
-        if (w0 + 32 == DT_TILE / 32) tile_total = running;  // the tile proper ends here, the overhang follows
-      }
-      if (lane == 0) pf[DT_WORDS] = (uint16_t)running;
-      __syncwarp();
-      // line breaks in front of the tile: look back over the tiles before it (aggregate / inclusive states)
-      unsigned long long before = 0;
-      if (lane == 0) {
-        volatile unsigned long long *st = A.tile_state;
-        if (t == 0) {
-          st[0] = DT_FLAG_INC | (unsigned long long)tile_total;
-        } else {
-          st[t] = DT_FLAG_AGG | (unsigned long long)tile_total;
-          __threadfence();
-          unsigned long long p = t;
-          while (true) {
-            --p;
-            unsigned long long v;
-            while (((v = st[p]) >> 62) == 0ull) {}
-            before += v & DT_VAL_MASK;
-            if ((v >> 62) == 2ull) break;
-          }
-          st[t] = DT_FLAG_INC | (before + tile_total);
-        }
-        __threadfence();
-        if (tile_total) atomicAdd(ctrl + 9, (unsigned long long)tile_total);  // census of the batch
-      }
-      before = __shfl_sync(0xffffffffu, before, 0);
-      // the tile's records: the line breaks whose global ordinal is 3 mod 4 have a header behind them
-      const uint32_t j0 = (3u - (uint32_t)(before & 3ull)) & 3u;
-      const uint32_t n_rec = tile_total > j0 ? (tile_total - j0 + 3u) / 4u : 0u;
-      if (lane == 0) {
-        if (n_rec) {  // end of the last complete record that ends in this tile: the batch's `consumed` is the maximum
-          uint32_t wq;
-          const uint32_t pe = nl_position(mk, pf, j0 + 4u * (n_rec - 1u), wq);
-          atomicMax(ctrl + 10, tile_lo + pe + 1ull);
-        }
-        M.before = before; M.tile_lo = tile_lo; M.n_rec = n_rec; M.j0 = j0; M.nload = nload; M.first = t == 0 ? 1u : 0u;
-        M.n_nl = running; M.at_end = tile_lo + nload >= A.n ? 1u : 0u;
-        s_next[b] = 0;
-        __threadfence_block();
-        mbar_arrive(&bar_ready[b]);
-      }
-      __syncwarp();
-    }
-  } else {
-    // ------------------------------------------------------------------ consumers
-    const int ctid = tid - 32, group = ctid / TRIM_THREADS;
-    uint32_t *ps_mine = ps_base + group * PS_ROWS_OF(A.pack_words) * TRIM_THREADS + (ctid & (TRIM_THREADS - 1));
-    FastCtx fc;
-    fc.s_eq = eq; fc.ps = ps_mine; fc.jump_ok = false; fc.rbase = 0;
-    for (uint32_t it = 0;; ++it) {
-      const int b = it % DT_NBUF;
-      const uint32_t par = (it / DT_NBUF) & 1u;
-      mbar_wait(&bar_ready[b], par);
-      const TileMeta M = s_meta[b];
-      if (M.n_rec == 0xFFFFFFFFu) break;
-      const uint32_t *mk = masks + b * DT_WORDS;
-      const uint16_t *pf = prefs + b * (DT_WORDS + 2);
-      const uint8_t *B = bufs + b * DT_LOAD - M.tile_lo;  // B[stream offset]
-      const uint32_t total = M.n_rec + M.first;
-      while (true) {
-        uint32_t c = 0;
-        if (lane == 0) c = atomicAdd(&s_next[b], 32u);
-        c = __shfl_sync(0xffffffffu, c, 0);
-        if (c >= total) break;
-        const uint32_t q = c + lane;
-        bool valid = q < total, far = false;
-        uint64_t r = 0;
-        uint4 ls = make_uint4(0, 0, 0, 0);
-        uint32_t nxt = 0;
-        if (valid) {
-          uint32_t p, w = 0;  // position of the line break in front of the record (none for record 0 of the stream)
-          if (M.first && q == 0) {
-            ls.x = A.skew;
-            p = 0xFFFFFFFFu;
-          } else {
-            const uint32_t j = M.j0 + 4u * (q - M.first);
-            p = nl_position(mk, pf, j, w);
-            ls.x = (uint32_t)M.tile_lo + p + 1u;
-            r = (M.before + j + 1ull) >> 2;
-          }
-          uint32_t e[4];
-          bool all = true;
-#pragma unroll
-          for (int k = 0; k < 4; ++k) {
-            if (all) {
-              if (p == 0xFFFFFFFFu && k == 0) {  // first line break of the stream
-                p = M.n_nl ? nl_position(mk, pf, 0u, w) : 0xFFFFFFFFu;
-              } else {
-                p = nl_next(mk, p, w);
-              }
-              all = p != 0xFFFFFFFFu;
-              e[k] = (uint32_t)M.tile_lo + p + 1u;
-            }
-          }
-          if (all) {
-            ls.y = e[0]; ls.z = e[1]; ls.w = e[2];
-            nxt = e[3];
-          } else if (M.at_end) {
-            valid = false;  // the stream ends inside this record: it is not a record of this batch
-          } else {
-            far = true;     // longer than the overhang: the whole-pipeline pass finds its lines
-            valid = false;
-          }
-          if ((valid || far) && r >= A.n_cap) {
-            atomicOr(ctrl + 2, 16ull);  // more records than the outputs have room for: the host repeats with the exact count
-            valid = far = false;
-          }
-          if (valid && A.line_start) {
-            *(uint4 *)(A.line_start + 4 * r) = ls;
-            A.line_start[4 * r + 4] = nxt;
-          }
-        }
-        const unsigned fm = __ballot_sync(0xffffffffu, far);
-        if (fm) {
-          unsigned long long fb = 0;
-          if (lane == __ffs(fm) - 1) fb = atomicAdd(ctrl + 5, (unsigned long long)__popc(fm));
-          fb = __shfl_sync(0xffffffffu, fb, __ffs(fm) - 1);
-          if (far) {
-            const unsigned long long at = fb + __popc(fm & ((1u << lane) - 1u));
-            if (at < A.ss.cap) {
-              SlowRec sr;
-              sr.r = (uint32_t)r; sr.x = ls.x; sr.y = 0; sr.z = 0; sr.w = 0; sr.nxt = 0; sr.pad0 = virtual_nl ? 1u : 0u; sr.pad1 = 0;
-              *(uint4 *)&A.ss.recs[at] = *(const uint4 *)&sr;
-              *((uint4 *)&A.ss.recs[at] + 1) = *((const uint4 *)&sr + 1);
-            } else {
-              atomicOr(ctrl + 2, 8ull);
-            }
-          }
-        }
-        process_record<32, true, 1, true>(valid, r, B, A.n, nullptr, A.win, A.key_off, A.keys, A.keys_cap, ctrl, A.ss, fc, ps_mine,
-                                          A.so, ls, nxt, A.il);
-        __syncwarp();
-      }
-      __syncwarp();
-      if (lane == 0) mbar_arrive(&bar_empty[b]);
-    }
-  }
+  process_record<MAXM, FAST, PASS, SPLIT>(valid, r, B, nbytes, line_start, win, key_off, keys, keys_cap, ctrl, d_slow, fc, ps_mine, so, ls, nxt, il);
   flush_stats(ctrl);
 }
 
@@ -1120,7 +744,7 @@ trim_dp_kernel(const DpEntry *__restrict__ entries, const uint32_t *__restrict__
     if (need_redo) slot_hi = slot_lo;
   }
   emit_record<true, 0>(valid, r, E, slot_lo, slot_hi, nullptr, true, w_start, w_stop, w_us, w_ue, w_words, false, win, key_off, keys, keys_cap,
-                       ctrl, SlowSink{nullptr, nullptr, 0}, make_uint4(0, 0, 0, 0), 0u, ps_mine, il);
+                       ctrl, nullptr, ps_mine, il);
   flush_stats(ctrl);
 }
 
@@ -1185,7 +809,7 @@ extern "C" int mirge_trim(mirge_ctx *ctx, const uint8_t *d_fastq, uint64_t nbyte
       // stage 1: every read up to the adapter modifier; exact adapter occurrences are settled here
       MIRGE_CUDA(ctx, cudaFuncSetAttribute(trim_kernel<32, true, 1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
       trim_kernel<32, true, 1, true><<<grid, TRIM_THREADS, smem + extra, stream>>>(d_fastq, nbytes, d_line_start, n_records, win, d_key_off,
-                                                                                 d_keys, keys_capacity_words, ctrl, smem, d_slow, so, il, pack_words, nullptr, 0u);
+                                                                                 d_keys, keys_capacity_words, ctrl, smem, d_slow, so, il, pack_words);
       MIRGE_LAUNCH_CHECK(ctx, "trim_kernel(stage 1)");
       // stages 2 and 3: the listed reads (counts live on the device: CTAs beyond the list exit at once)
       const size_t dp_smem = extra + (size_t)TRIM_THREADS * (sizeof(DpEntry) + 4 + 2);
@@ -1200,7 +824,7 @@ extern "C" int mirge_trim(mirge_ctx *ctx, const uint8_t *d_fastq, uint64_t nbyte
       // pass 1: every read; adapter searches that need cost columns are deferred to the list d_slow
       trim_kernel<32, true, 1, false><<<grid, TRIM_THREADS, smem + extra, stream>>>(d_fastq, nbytes, d_line_start, n_records, win,
                                                                                   d_key_off, d_keys, keys_capacity_words, ctrl, smem,
-                                                                                  d_slow, so, il, pack_words, nullptr, 0u);
+                                                                                  d_slow, so, il, pack_words);
       MIRGE_LAUNCH_CHECK(ctx, "trim_kernel(pass 1)");
     }
     // pass 2: the reads left over (whole pipeline per read, from the global stream; grid-stride over the list)
@@ -1209,114 +833,17 @@ extern "C" int mirge_trim(mirge_ctx *ctx, const uint8_t *d_fastq, uint64_t nbyte
     unsigned grid2 = split ? grid / 4 + 1 : grid / 16 + 1;
     if (grid2 > (unsigned)ctx->sm_count * (split ? 64u : 8u)) grid2 = (unsigned)ctx->sm_count * (split ? 64u : 8u);
     trim_kernel<32, true, 2, false><<<grid2, TRIM_THREADS, extra, stream>>>(d_fastq, nbytes, d_line_start, n_records, win, d_key_off,
-                                                                          d_keys, keys_capacity_words, ctrl, 0u, d_slow, so, il, pack_words, nullptr, 0u);
+                                                                          d_keys, keys_capacity_words, ctrl, 0u, d_slow, so, il, pack_words);
   } else if (ctx->max_adapter_len <= 32) {
     MIRGE_CUDA(ctx, cudaFuncSetAttribute(trim_kernel<32, false, 0, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024));
     trim_kernel<32, false, 0, false><<<grid, TRIM_THREADS, smem, stream>>>(d_fastq, nbytes, d_line_start, n_records, win, d_key_off,
-                                                                           d_keys, keys_capacity_words, ctrl, smem, nullptr, so, il, 8, nullptr, 0u);
+                                                                           d_keys, keys_capacity_words, ctrl, smem, nullptr, so, il, 8);
   } else {
     MIRGE_CUDA(ctx, cudaFuncSetAttribute(trim_kernel<64, false, 0, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024));
     trim_kernel<64, false, 0, false><<<grid, TRIM_THREADS, smem, stream>>>(d_fastq, nbytes, d_line_start, n_records, win, d_key_off,
-                                                                           d_keys, keys_capacity_words, ctrl, smem, nullptr, so, il, 8, nullptr, 0u);
+                                                                           d_keys, keys_capacity_words, ctrl, smem, nullptr, so, il, 8);
   }
   MIRGE_LAUNCH_CHECK(ctx, "trim_kernel");
-  return MIRGE_OK;
-}
-
-// ---- fused path: scratch layout [tile states u64[n_tiles]][whole-pipeline records 32 B x slow_cap][stage-3 list u32[n_cap]]
-//      [DpEntry[n_cap]][packed text u32[MAX_PACK_WORDS][n_cap]]
-static uint64_t dt_tiles(uint64_t nbytes) { return (nbytes + 16) / DT_TILE + 1; }
-static uint64_t dt_slow_cap(uint64_t n_cap) { return n_cap; }  // every record may need the whole-pipeline pass (reads full of N)
-
-extern "C" int mirge_digest_fused_ok(const mirge_ctx *ctx) {
-  if (!ctx || !ctx->params_set) return 0;
-  return ctx->fast_ok && ctx->split_ok && ctx->trim_mode == 0;
-}
-
-extern "C" uint64_t mirge_digest_scratch_bytes(uint64_t nbytes, uint64_t n_cap) {
-  const uint64_t n = n_cap ? n_cap : 1;
-  return align16(8 * dt_tiles(nbytes)) + align16(sizeof(SlowRec) * dt_slow_cap(n)) + align16(4 * n) + align16(sizeof(DpEntry) * n) +
-         align16(4ull * MAX_PACK_WORDS * n) + 64;
-}
-
-extern "C" int mirge_digest_tiles(mirge_ctx *ctx, const uint8_t *d_fastq, uint64_t nbytes, int is_final, uint64_t n_cap,
-                                  uint32_t *d_line_start, uint16_t *d_win, uint32_t *d_key_off, uint32_t *d_keys,
-                                  uint64_t keys_capacity_words, uint64_t *d_trim_ctrl, void *d_scratch, uint64_t *d_ins,
-                                  uint64_t ins_capacity, void *stream_) {
-  if (!ctx) return MIRGE_ERR_ARG;
-  if (!ctx->params_set) MIRGE_FAIL(ctx, MIRGE_ERR_ARG, "digest: mirge_set_trim_params has not been called");
-  if (!mirge_digest_fused_ok(ctx)) MIRGE_FAIL(ctx, MIRGE_ERR_ARG, "digest: the fused path needs 3' adapters of <= 32 nt with indels (use mirge_trim)");
-  if (nbytes == 0) return MIRGE_OK;
-  if (!d_fastq || !d_keys || !d_trim_ctrl || !d_scratch || n_cap == 0) MIRGE_FAIL(ctx, MIRGE_ERR_ARG, "digest: null buffer");
-  if (nbytes > 0xFFFFFF00ull) MIRGE_FAIL(ctx, MIRGE_ERR_ARG, "digest: batch larger than 4 GiB - 256");
-  if (!d_win != !d_key_off) MIRGE_FAIL(ctx, MIRGE_ERR_ARG, "digest: d_win and d_key_off go together");
-  if (!d_key_off && !d_ins) MIRGE_FAIL(ctx, MIRGE_ERR_ARG, "digest: neither per-slot outputs nor an insert list requested");
-  if (d_ins && (ins_capacity < n_cap * (uint64_t)trim_slots_of(&ctx->params) || ((uintptr_t)d_ins & 7)))
-    MIRGE_FAIL(ctx, MIRGE_ERR_ARG, "digest: bad insert list");
-  if (((uintptr_t)d_line_start & 15) || ((uintptr_t)d_win & 7) || ((uintptr_t)d_scratch & 15)) MIRGE_FAIL(ctx, MIRGE_ERR_ARG, "digest: misaligned buffer");
-  if (n_cap >= 0x80000000ull || n_cap * (uint64_t)trim_slots_of(&ctx->params) >= MAX_LIST_ITEMS)
-    MIRGE_FAIL(ctx, MIRGE_ERR_ARG, "digest: more than 2^28 emission slots in one batch (use smaller batches)");
-  cudaStream_t stream = (cudaStream_t)stream_;
-  MIRGE_CUDA(ctx, cudaSetDevice(ctx->device));
-  const uint32_t skew = (uint32_t)((uintptr_t)d_fastq & 15);
-  DigestTilesArgs A;
-  A.fq = d_fastq - skew;
-  A.n = nbytes + skew;
-  A.skew = skew;
-  A.is_final = is_final ? 1u : 0u;
-  A.n_tiles = A.n / DT_TILE + 1;
-  uint8_t *sc = (uint8_t *)d_scratch;
-  A.tile_state = (unsigned long long *)sc;
-  sc += align16(8 * dt_tiles(nbytes));
-  A.ss.r_list = nullptr;
-  A.ss.recs = (SlowRec *)sc;
-  A.ss.cap = dt_slow_cap(n_cap);
-  sc += align16(sizeof(SlowRec) * A.ss.cap);
-  uint32_t *d_redo = (uint32_t *)sc;
-  sc += align16(4 * n_cap);
-  A.so.entries = (DpEntry *)sc;
-  sc += align16(sizeof(DpEntry) * n_cap);
-  A.so.pk = (uint32_t *)sc;
-  A.so.cap = n_cap;
-  A.line_start = d_line_start;
-  A.n_cap = (uint32_t)n_cap;
-  A.win = (ushort4 *)d_win;
-  A.key_off = d_key_off;
-  A.keys = d_keys;
-  A.keys_cap = keys_capacity_words;
-  A.ctrl = (unsigned long long *)d_trim_ctrl;
-  A.il = InsList{(uint2 *)d_ins, d_ins ? ins_capacity : 0};
-  // packed-read rows: 8 words cover reads of up to 128 bases (an average record of <= 264 bytes says they are)
-  const uint64_t avg = (nbytes + n_cap - 1) / n_cap;
-  A.pack_words = avg <= 2 * 112 + 40 ? 8 : MAX_PACK_WORDS;
-  MIRGE_CUDA(ctx, cudaMemsetAsync(A.tile_state, 0, 8 * A.n_tiles, stream));
-  const size_t rows = (size_t)PS_ROWS_OF(A.pack_words) * TRIM_THREADS * 4;
-  const size_t dt_smem = (size_t)DT_NBUF * DT_LOAD + (size_t)DT_NBUF * DT_WORDS * 4 + (size_t)DT_NBUF * (DT_WORDS + 2) * 2 +
-                         (size_t)ctx->params.n_adapters * 1024 + DT_GROUPS * rows;
-  MIRGE_CUDA(ctx, cudaFuncSetAttribute(digest_tiles_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-  int per_sm = 0;
-  MIRGE_CUDA(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, digest_tiles_kernel, DT_THREADS, dt_smem));
-  if (per_sm < 1) MIRGE_FAIL(ctx, MIRGE_ERR_CUDA, "digest: the fused kernel does not fit an SM");
-  uint64_t grid = (uint64_t)ctx->sm_count * per_sm;  // persistent: every CTA resident, tiles by ticket
-  if (grid > A.n_tiles) grid = A.n_tiles;
-  digest_tiles_kernel<<<(unsigned)grid, DT_THREADS, dt_smem, stream>>>(A);
-  MIRGE_LAUNCH_CHECK(ctx, "digest_tiles_kernel");
-  // stages 2 and 3 and the whole-pipeline pass, list-driven (counts live on the device: CTAs beyond a list exit at once)
-  const unsigned lgrid = (unsigned)((n_cap + TRIM_THREADS - 1) / TRIM_THREADS);
-  const size_t extra = (size_t)ctx->params.n_adapters * 1024 + rows;
-  const size_t dp_smem = extra + (size_t)TRIM_THREADS * (sizeof(DpEntry) + 4 + 2);
-  trim_dp_kernel<true><<<lgrid, TRIM_THREADS, dp_smem, stream>>>(A.so.entries, A.so.pk, A.so.cap, d_redo, A.win, d_key_off, d_keys,
-                                                                 keys_capacity_words, A.ctrl, A.il, A.pack_words);
-  MIRGE_LAUNCH_CHECK(ctx, "trim_dp_kernel(stage 2)");
-  trim_dp_kernel<false><<<lgrid, TRIM_THREADS, dp_smem, stream>>>(A.so.entries, A.so.pk, A.so.cap, d_redo, A.win, d_key_off, d_keys,
-                                                                  keys_capacity_words, A.ctrl, A.il, A.pack_words);
-  MIRGE_LAUNCH_CHECK(ctx, "trim_dp_kernel(stage 3)");
-  unsigned grid2 = lgrid / 4 + 1;
-  if (grid2 > (unsigned)ctx->sm_count * 64u) grid2 = (unsigned)ctx->sm_count * 64u;
-  trim_kernel<32, true, 2, false><<<grid2, TRIM_THREADS, extra, stream>>>(A.fq, A.n, d_line_start, n_cap, A.win, d_key_off, d_keys,
-                                                                        keys_capacity_words, A.ctrl, 0u, nullptr, A.so, A.il,
-                                                                        A.pack_words, A.ss.recs, (uint32_t)n_cap);
-  MIRGE_LAUNCH_CHECK(ctx, "trim_kernel(whole-pipeline pass)");
   return MIRGE_OK;
 }
 

@@ -296,10 +296,6 @@ class DigestEngine:
         self.E = dev.slots
         self.trim_mode = 0  # 0 = automatic kernel choice, 1 = always the generic full-DP kernel
         self.INPLACE_MIN_NEW = float(os.environ.get("MIRGE_B200_INPLACE_MIN_NEW", "0.25"))
-        # single-pass tokenise + stage 1 (bulk-copy fed persistent kernel) where it applies; off by default: measured
-        # slower than tokenise -> line index -> stage 1 on the B200 (profiles/README.md), kept selectable
-        self.fused = os.environ.get("MIRGE_B200_FUSED", "0") == "1"
-        self._avg_record = None  # bytes per record of the last batch (record bound of the fused kernel)
         dev.check(dev.lib.mirge_trim_mode(dev.ctx, 0))
         self.stats = {"records": 0, "bytes": 0, "emitted": 0, "key_words": 0, "deferred": 0, "dp_reads": 0, "dp_redo": 0}  # running totals (bench.py rooflines)
 
@@ -309,106 +305,13 @@ class DigestEngine:
 
     def trim_batch(self, buf: torch.Tensor, nbytes: int, is_final: bool, keep: bool = True,
                    table: Optional["CollapseTable"] = None) -> BatchResult:
-        """Tokenise + trim buf[:nbytes] (uint8, device).  Returns the device arrays the collapse consumes (and the
+        """tokenise -> line index -> trim of buf[:nbytes] (uint8, device), with every kernel choice of mirge_trim (split
+        bit-parallel pipeline, generic full DP, qiagen UMIs).  Returns the device arrays the collapse consumes (and the
         parity tests read).  With ``table`` the packed keys are written straight into that table's arena (zero-copy
-        collapse); otherwise into a batch buffer.  The fused single-pass kernel runs where it applies
-        (mirge_digest_fused_ok), the tokenise -> line index -> trim path otherwise."""
+        collapse); otherwise into a batch buffer."""
         if nbytes == 0:
             return BatchResult(0, 0, 0, 0)
-        if self.fused and self.trim_mode == 0 and self.dev.lib.mirge_digest_fused_ok(self.dev.ctx):
-            br = self._trim_batch_fused(buf, nbytes, is_final, keep, table)
-            if br is not None:
-                return br
-        return self._trim_batch_two_pass(buf, nbytes, is_final, keep, table)
-
-    def _trim_batch_fused(self, buf, nbytes, is_final, keep, table) -> Optional[BatchResult]:
-        """One pass over the bytes: mirge_digest_tiles.  None: the batch needs the two-pass path (too many records for
-        the whole-pipeline list)."""
         d, lib, E = self.dev, self.dev.lib, self.E
-        st = d.stream()
-        skew = int(buf.data_ptr()) & 15
-        if self._avg_record is None:
-            # the kernel needs a bound on the number of records: the first 64 KB of the first batch give the scale
-            head = buf[: min(nbytes, 1 << 16)].cpu().numpy()
-            lines = int((head == 10).sum())
-            self._avg_record = max(head.size / max(lines / 4.0, 1.0), 8.0)
-        n_cap = int(nbytes / self._avg_record * 1.15) + 1024
-        if table is not None and table.new_frac < self.INPLACE_MIN_NEW:
-            table = None  # repeats dominate: batch key buffer + copying insert keeps the arena tight
-        base_words = 0
-        if table is not None:
-            table.check()
-            base_words = table.arena_used
-        cap = None
-        for attempt in range(6):
-            line_start = d.empty(4 * n_cap + 4, torch.int32) if keep else None
-            win = d.empty(n_cap * E * 4, torch.int16) if keep else None
-            key_off = d.empty(n_cap * E, torch.int32) if keep else None
-            ins = d.empty(n_cap * E, torch.int64)
-            scratch = d.empty(lib.mirge_digest_scratch_bytes(nbytes, n_cap), torch.uint8)
-            if cap is None:
-                cap = E * (2 * n_cap + nbytes // 24) + 4096
-            ctrl = d.zeros(16, torch.int64)
-            if table is not None:
-                table.reserve(0, cap)
-                keys = table.arena
-                ctrl[0:1].fill_(base_words)
-                cap_abs = int(table.arena.numel())
-            else:
-                keys = d.empty(cap, torch.int32)
-                cap_abs = cap
-            with d.timed("trim"):
-                d.check(lib.mirge_digest_tiles(d.ctx, _ptr(buf), nbytes, 1 if is_final else 0, n_cap, _ptr(line_start), _ptr(win),
-                                               _ptr(key_off), _ptr(keys), cap_abs, _ptr(ctrl), _ptr(scratch), _ptr(ins), n_cap * E, st))
-            d.launches += 4
-            c = ctrl.cpu().numpy().view(np.uint64)
-            words_used, n_items = int(c[0]) & ((1 << 36) - 1), int(c[0]) >> 36
-            flags, total_lines = int(c[2]), int(c[9])
-            if flags & 16:  # more records than estimated: the census is exact, repeat with it
-                n_cap = total_lines // 4 + 16
-                continue
-            if flags & 8:
-                return None
-            if flags & 1:
-                rec = int(np.uint64(~c[3]))
-                raise FastqFormatError("FASTQ format error in record %d of the batch (header must start with '@', "
-                                       "line 3 with '+', sequence and qualities must have equal length)" % rec)
-            if flags & 4:
-                raise MirgeError("read longer than %d bases is not supported" % abi.MAX_READ_LEN)
-            if flags & 2:
-                if attempt >= 4:
-                    raise CapacityError("trim: key buffer overflow")
-                cap = E * (n_cap + nbytes // 2 + nbytes // 32 + 64) + 4096  # worst case: every base an exception
-                continue
-            break
-        else:
-            raise CapacityError("digest: the record bound did not settle")
-        if is_final:
-            if total_lines % 4:
-                raise FastqFormatError("FASTQ format error: %d lines is not a multiple of 4 (premature end of file)" % total_lines)
-            n, used = total_lines // 4, nbytes
-        else:
-            n = total_lines // 4
-            used = int(c[10]) - skew if n else 0
-        if n:
-            self._avg_record = max(used / n, 8.0)
-        self.stats["deferred"] += int(c[5])
-        self.stats["dp_reads"] += int(c[6])
-        self.stats["dp_redo"] += int(c[7])
-        if keep:
-            line_start, win, key_off = line_start[: 4 * n + 4], win[: n * E * 4], key_off[: n * E]
-        if table is not None:
-            table.arena_used = words_used
-            table.ctrl[0:1].fill_(table.arena_used)
-            return BatchResult(n, used, int(c[1]), int(c[4]), line_start, win, key_off, None, True, words_used - base_words, ins, n_items)
-        return BatchResult(n, used, int(c[1]), int(c[4]), line_start, win, key_off, keys, False, words_used, ins, n_items)
-
-    def _trim_batch_two_pass(self, buf: torch.Tensor, nbytes: int, is_final: bool, keep: bool = True,
-                             table: Optional["CollapseTable"] = None) -> BatchResult:
-        """tokenise -> line index -> trim: every kernel choice of mirge_trim (generic full DP, unsplit, qiagen UMIs)."""
-        d, lib, E = self.dev, self.dev.lib, self.E
-        if nbytes == 0:
-            return BatchResult(0, 0, 0, 0)
         st = d.stream()
         scratch = d.empty(lib.mirge_tokenise_scratch_bytes(nbytes), torch.uint8)
         n_rec, consumed = C.c_uint64(0), C.c_uint64(0)

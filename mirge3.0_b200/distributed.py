@@ -3,10 +3,11 @@
 The path shards naturally (SURVEY.md section 8e): FASTQ chunks / samples are split across ranks, every
 rank collapses locally, and exactly one exchange makes each rank the owner of a disjoint slice of the
 unique sequences: records (count, packed key) are partitioned by hash64(centre sequence) mod world
-(kernel: mirge_partition_plan), packed per destination (mirge_partition_pack), moved with a single
-all-to-all, and merged into the owner's table (mirge_collapse_merge).  With UMIs the centre (UMI flanks
-removed) is hashed, so both UMI levels are owner-local.  Libraries are replicated; annotation then runs on
-the owner's slice with no further communication.  The reference has no counterpart: its only
+(kernel: mirge_partition_plan), packed per destination (mirge_partition_totals + mirge_partition_scatter),
+moved with a single all-to-all straight into the owner's arena, and merged into the owner's table there
+(mirge_collapse_merge_inplace).  With UMIs the centre (UMI flanks removed) is hashed, so both UMI levels
+are owner-local.  Libraries are replicated; annotation then runs on the owner's slice with no further
+communication.  The reference has no counterpart: its only
 parallelism is a fork pool whose results are merged by one Python loop (digest.py:139-163)."""
 from __future__ import annotations
 

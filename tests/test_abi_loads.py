@@ -8,7 +8,9 @@ import mirge_b200
 from mirge_b200 import abi
 
 
-def test_library_exports_every_declared_symbol():
+def test_library_matches_declared_abi():
+    """Every symbol the header declares is exported and bound, and library, header and bindings agree on the ABI
+    version."""
     import __graft_entry__ as g
 
     g.build()
@@ -18,7 +20,8 @@ def test_library_exports_every_declared_symbol():
     assert declared == set(abi.SYMBOLS), declared ^ set(abi.SYMBOLS)
     for name in declared:
         assert getattr(lib, name) is not None
-    assert lib.mirge_abi_version() == abi.ABI_VERSION == 3
+    hdr_version = int(re.search(r"#define MIRGE_ABI_VERSION (\d+)", hdr).group(1))
+    assert lib.mirge_abi_version() == abi.ABI_VERSION == hdr_version == 4
 
 
 def test_struct_sizes_match_header():

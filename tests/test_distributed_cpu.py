@@ -1,6 +1,6 @@
 """Host-side logic of the multi-GPU path on CPU (gloo, world_size 2): sharding + the variable-size
 record all-to-all (mirge_b200.distributed.exchange_records).  Records are built by the oracle's
-collapse here; on GPUs the same plumbing moves records packed by mirge_partition_pack."""
+collapse here; on GPUs the same plumbing moves records packed by mirge_partition_scatter."""
 import os
 import socket
 import zlib

@@ -1,4 +1,4 @@
-"""Host check of the tokeniser's newline-mask arithmetic (csrc/common.cuh::newline_mask, shared by tokenise.cu and the fused kernel of trim.cu; the kernel replaces the
+"""Host check of the tokeniser's newline-mask arithmetic (csrc/common.cuh::newline_mask, used by tokenise.cu; the kernel replaces the
 line splitting of dnaio's FastqIter, reference call site mirge/libs/digest.py:324) against a plain byte compare.
 It is a pure integer trick, so it is restated with numpy and swept over random words: any byte values, dense
 newlines, bytes >= 128."""
