@@ -331,6 +331,13 @@ int mirge_shard_scatter(mirge_ctx *ctx, const uint32_t *d_keys, const uint64_t *
                         uint32_t *d_out_keys, void *stream);
 int mirge_shard_rebase(mirge_ctx *ctx, uint64_t *d_items, uint32_t n_parts, const uint64_t *item_counts,
                        const uint64_t *key_bases, void *stream);
+/* mirge_shard_scatter_centre: mirge_shard_scatter with the owner hashed from the key's centre, the key without its
+ * umi5 leading and umi3 trailing bases -- the owner mirge_partition_plan gives the same key with the same umi5 / umi3.
+ * All first-level keys of one centre go to one rank (UMI runs: the second level is owner-local).  The whole key is
+ * copied to the region; regions, cursors and the overflow rule are those of mirge_shard_scatter. */
+int mirge_shard_scatter_centre(mirge_ctx *ctx, const uint32_t *d_keys, const uint64_t *d_ins, uint64_t n_items,
+                               uint32_t n_parts, int umi5, int umi3, uint32_t cap_items, uint32_t cap_words,
+                               uint64_t *d_cursors, uint64_t *d_out_items, uint32_t *d_out_keys, void *stream);
 
 /* ---- stage 3: annotation rounds (bwtAlign, manifoldAlign.py:68-146) ------------------------ */
 /* 16-mer (zero padded, truncated at reference ends / ambiguous bases) of every base position:

@@ -153,6 +153,10 @@ SYMBOLS = {
     "mirge_partition_scatter": (C.c_int, [_P, C.POINTER(Table), _P, _P, _P, _P, _U64, C.c_uint32, _P, _P, _P, _P]),
     "mirge_shard_scatter": (C.c_int, [_P, _P, _P, _U64, C.c_uint32, C.c_uint32, C.c_uint32, _P, _P, _P, _P]),
     "mirge_shard_rebase": (C.c_int, [_P, _P, C.c_uint32, _PU64, _PU64, _P]),
+    "mirge_shard_scatter_centre": (
+        C.c_int,
+        [_P, _P, _P, _U64, C.c_uint32, C.c_int, C.c_int, C.c_uint32, C.c_uint32, _P, _P, _P, _P],
+    ),
     "mirge_lib_kmers": (C.c_int, [_P, C.POINTER(Library), _P, _P, _P]),
     "mirge_lib_filter": (C.c_int, [_P, _P, _P, C.c_uint32, C.c_uint32, _P, _P]),
     "mirge_lib_filter16": (C.c_int, [_P, _P, _P, C.c_uint32, C.c_uint32, _P, _P]),

@@ -850,10 +850,14 @@ __device__ __forceinline__ uint32_t owner_of(uint64_t h, uint32_t n_parts) {
   return (uint32_t)(mix64(h ^ 0x5851F42D4C957F2Dull) % n_parts);
 }
 
+// CENTRE: the owner hashes the key without its f / b UMI flanks (slice_key), which is the owner partition_plan_kernel
+// gives the same key: all first-level keys of one centre meet at one rank, so the UMI second level is owner-local.  The
+// whole key still travels (the owner's first-level table needs it).
+template <bool CENTRE>
 __global__ void __launch_bounds__(COL_THREADS)
 shard_scatter_kernel(const uint32_t *__restrict__ keys, const uint2 *__restrict__ ins, uint64_t n, uint32_t n_parts,
                      uint32_t cap_items, uint32_t cap_words, unsigned long long *__restrict__ cursors,
-                     uint2 *__restrict__ out_items, uint32_t *__restrict__ out_keys) {
+                     uint2 *__restrict__ out_items, uint32_t *__restrict__ out_keys, int f, int b) {
   // (two 32-bit counters per owner: item slot and key space of an item are handed out independently -- the item
   // carries its key's offset -- and 32-bit shared-memory atomics are native, 64-bit ones a compare-and-swap loop)
   __shared__ uint32_t s_items[MAX_PARTS], s_words[MAX_PARTS], s_bi[MAX_PARTS], s_bw[MAX_PARTS], s_ok[MAX_PARTS];
@@ -873,7 +877,13 @@ shard_scatter_kernel(const uint32_t *__restrict__ keys, const uint2 *__restrict_
     off[it] = item.x;
     add[it] = item.y;
     nw[it] = w;
-    const uint32_t d = owner_of(hash_key(key, w), n_parts);
+    uint32_t d;
+    if (CENTRE) {
+      uint32_t buf[MAX_KEY_WORDS];
+      d = owner_of(hash_key(buf, slice_key(key, f, b, buf)), n_parts);
+    } else {
+      d = owner_of(hash_key(key, w), n_parts);
+    }
     dst[it] = d;
     // item slots: one atomic per group of lanes with the same owner
     const unsigned peers = __match_any_sync(__activemask(), d);
@@ -909,22 +919,38 @@ shard_scatter_kernel(const uint32_t *__restrict__ keys, const uint2 *__restrict_
   }
 }
 
-extern "C" int mirge_shard_scatter(mirge_ctx *ctx, const uint32_t *d_keys, const uint64_t *d_ins, uint64_t n_items, uint32_t n_parts,
-                                   uint32_t cap_items, uint32_t cap_words, uint64_t *d_cursors, uint64_t *d_out_items,
-                                   uint32_t *d_out_keys, void *stream_) {
+template <bool CENTRE>
+static int shard_scatter(mirge_ctx *ctx, const uint32_t *d_keys, const uint64_t *d_ins, uint64_t n_items, uint32_t n_parts,
+                         int f, int b, uint32_t cap_items, uint32_t cap_words, uint64_t *d_cursors, uint64_t *d_out_items,
+                         uint32_t *d_out_keys, void *stream_) {
   if (!ctx) return MIRGE_ERR_ARG;
   if (!d_cursors || n_parts == 0 || n_parts > MAX_PARTS) MIRGE_FAIL(ctx, MIRGE_ERR_ARG, "shard_scatter: 1..%d owners", MAX_PARTS);
+  if (f < 0 || b < 0) MIRGE_FAIL(ctx, MIRGE_ERR_ARG, "shard_scatter: negative UMI length");
   cudaStream_t stream = (cudaStream_t)stream_;
   MIRGE_CUDA(ctx, cudaSetDevice(ctx->device));
   MIRGE_CUDA(ctx, cudaMemsetAsync(d_cursors, 0, n_parts * sizeof(uint64_t), stream));
   if (n_items == 0) return MIRGE_OK;
   if (!d_keys || !d_ins || !d_out_items || !d_out_keys) MIRGE_FAIL(ctx, MIRGE_ERR_ARG, "shard_scatter: null buffer");
   const uint64_t per_cta = (uint64_t)COL_THREADS * XS_ITEMS;
-  shard_scatter_kernel<<<(unsigned)((n_items + per_cta - 1) / per_cta), COL_THREADS, 0, stream>>>(
+  shard_scatter_kernel<CENTRE><<<(unsigned)((n_items + per_cta - 1) / per_cta), COL_THREADS, 0, stream>>>(
       d_keys, (const uint2 *)d_ins, n_items, n_parts, cap_items, cap_words, (unsigned long long *)d_cursors, (uint2 *)d_out_items,
-      d_out_keys);
+      d_out_keys, f, b);
   MIRGE_LAUNCH_CHECK(ctx, "shard_scatter_kernel");
   return MIRGE_OK;
+}
+
+extern "C" int mirge_shard_scatter(mirge_ctx *ctx, const uint32_t *d_keys, const uint64_t *d_ins, uint64_t n_items, uint32_t n_parts,
+                                   uint32_t cap_items, uint32_t cap_words, uint64_t *d_cursors, uint64_t *d_out_items,
+                                   uint32_t *d_out_keys, void *stream_) {
+  return shard_scatter<false>(ctx, d_keys, d_ins, n_items, n_parts, 0, 0, cap_items, cap_words, d_cursors, d_out_items, d_out_keys,
+                              stream_);
+}
+
+extern "C" int mirge_shard_scatter_centre(mirge_ctx *ctx, const uint32_t *d_keys, const uint64_t *d_ins, uint64_t n_items,
+                                          uint32_t n_parts, int umi5, int umi3, uint32_t cap_items, uint32_t cap_words,
+                                          uint64_t *d_cursors, uint64_t *d_out_items, uint32_t *d_out_keys, void *stream_) {
+  return shard_scatter<true>(ctx, d_keys, d_ins, n_items, n_parts, umi5, umi3, cap_items, cap_words, d_cursors, d_out_items,
+                             d_out_keys, stream_);
 }
 
 // Receive side: the items of the n_parts sources lie back to back (source s = items [item_end[s-1], item_end[s])) and

@@ -263,15 +263,27 @@ def digest_sample(eng: DigestEngine, source, table: CollapseTable, first_level: 
 def _write_umi_csv(path: str, first: CollapseTable, ids: np.ndarray, counts: np.ndarray, umi: Tuple[int, int], min_len: int):
     """<sample>_umiCounts.csv (digest.py:185-205): header + one row per first-level key whose centre
     passes the length filter; opened in append mode like the reference (quirk 4)."""
-    keys = first.export_keys()
+    write_umi_csv_rows(path, umi_csv_rows(first.export_keys()[ids], counts, umi, min_len))
+
+
+def umi_csv_rows(keys: np.ndarray, counts: np.ndarray, umi: Tuple[int, int], min_len: int) -> str:
+    """The rows of <sample>_umiCounts.csv for first-level keys ``keys`` ('S' array) with their counts: centres shorter
+    than ``min_len`` are left out."""
     f_, b_ = umi
+    rows = []
+    for k, c in zip(keys.tolist(), counts.tolist()):
+        s = k.decode("latin-1")
+        center = s[f_:-b_] if int(b_) != 0 else s[f_:]
+        if len(center) >= int(min_len):
+            rows.append(s[:f_] + s[-b_:] + "," + center + "," + str(c) + "\n")  # UMIParser incl. the b == 0 quirk
+    return "".join(rows)
+
+
+def write_umi_csv_rows(path: str, rows: str):
+    """Header + ``rows`` appended to <sample>_umiCounts.csv (append mode like the reference, quirk 4)."""
     with open(path, "a+") as fh:
         fh.write("UMISeq" + "," + "transcriptSeq," + "UMICounts" + "\n")
-        for i, c in zip(ids.tolist(), counts.tolist()):
-            s = keys[i].decode("latin-1")
-            center = s[f_:-b_] if int(b_) != 0 else s[f_:]
-            if len(center) >= int(min_len):
-                fh.write(s[:f_] + s[-b_:] + "," + center + "," + str(c) + "\n")  # UMIParser incl. the b == 0 quirk
+        fh.write(rows)
 
 
 def _no_keys():
@@ -457,12 +469,17 @@ def baking(args, inFileArray, inFileBaseArray, workDir, device: Optional[Device]
 
 def write_tcf(workDir, base, table: CollapseTable, res: SampleResult):
     """``<sample>.trim.collapse.fa`` (digest.py:226-235): the sample's sequences by descending count (stable)."""
-    keys = table.export_keys()
-    order = np.argsort(-res.counts, kind="stable")
+    write_tcf_rows(workDir, base, table.export_keys()[res.ids], res.counts)
+
+
+def write_tcf_rows(workDir, base, keys: np.ndarray, counts: np.ndarray):
+    """``<sample>.trim.collapse.fa`` from the sample's sequences ``keys`` ('S' array) and their counts: by descending
+    count (stable)."""
+    order = np.argsort(-counts, kind="stable")
     with open(Path(workDir) / (str(base) + ".trim.collapse.fa"), "w") as fo:
         for hc, j in enumerate(order.tolist(), 1):
-            fo.write(">seq" + str(hc) + "_" + str(int(res.counts[j])) + "\n")
-            fo.write(keys[res.ids[j]].decode("latin-1") + "\n")
+            fo.write(">seq" + str(hc) + "_" + str(int(counts[j])) + "\n")
+            fo.write(keys[j].decode("latin-1") + "\n")
 
 
 def _write_histograms(workDir, df: pd.DataFrame, results: List[SampleResult], names: List[str], umi):

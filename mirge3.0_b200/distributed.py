@@ -230,29 +230,33 @@ class ShardedCollapse:
     sharding BEFORE the collapse.  Per batch of a rank's reads:
 
         pack      the batch's insert list (what the trim kernels wrote: packed keys + (key offset, count) items) is cut
-                  by owner = hash(key) mod world into fixed-capacity regions (mirge_shard_scatter);
+                  by owner = hash(key) mod world into fixed-capacity regions (mirge_shard_scatter; with ``umi`` = (f, b)
+                  the hash of the key's centre, mirge_shard_scatter_centre, so the UMI second level is owner-local);
         sizes     one all-gather of the per-owner (items, words) tells every rank what it will receive; the flag that
                   rides along says whether the rank has more input, so ranks with fewer batches keep joining rounds;
-        exchange  two all-to-alls with exact sizes (items; key words straight into the end of the owner's arena);
+        exchange  two all-to-alls with exact sizes (items; key words straight into the end of the owner's arena -- or,
+                  once repeats dominate the owner's table, into a buffer of the round: place / place_copy);
         insert    key offsets made absolute (mirge_shard_rebase), then the single-GPU collapse
-                  (mirge_collapse_insert_list, keys in place).
+                  (mirge_collapse_insert_list: keys in place, or copying only the new keys out of the round's buffer,
+                  the single-GPU rule of DigestEngine.trim_batch, so the arena grows with unique sequences: insert /
+                  insert_copy).
 
     The rounds are software-pipelined: while round k is packed, round k - 1 is on the wire and round k - 2 is inserted.
     Collectives run on side streams (under the next batch's trim kernels; sizes and data on separate communicators, so
     a round's few bytes of sizes never queue behind the previous round's data) and the sizes come back through pinned
     memory: the launch stream never waits for the host or the network.  Every emitted key is inserted exactly once,
     into the table of the rank that owns it: there is no local table and no drain / sort / merge of unique sequences
-    (exchange_and_merge above, still the path for samples dealt whole to ranks: baking_sharded).  Owner tables, key ids
-    and the annotation that follows are the single-GPU ones.
+    (exchange_and_merge above).  Owner tables, key ids and the annotation that follows are the single-GPU ones.
 
         more = True
         for every local batch:  more = sc.round(table, br, has_more_input)
         sc.drain_rounds(table, more)          # join the other ranks' remaining rounds, insert the last arrivals
     """
 
-    def __init__(self, eng, world: int, group=None, overlap: bool = True, slack: float = 1.2):
+    def __init__(self, eng, world: int, group=None, overlap: bool = True, slack: float = 1.2, umi=None):
         self.eng, self.dev = eng, eng.dev
         self.world, self.group = int(world), group
+        self.umi = (int(umi[0]), int(umi[1])) if umi is not None else None
         self.slack = float(slack)
         self.overlap = bool(overlap)
         self.size_group = group
@@ -298,9 +302,14 @@ class ShardedCollapse:
             if br.in_place:
                 raise RuntimeError("ShardedCollapse.pack: the batch must be trimmed into a batch buffer (table=None)")
             src_keys = br.keys
+        src_ins = _ptr(br.ins if n_items else None)
         with d.timed("shard_pack"):
-            d.check(d.lib.mirge_shard_scatter(d.ctx, _ptr(src_keys), _ptr(br.ins if n_items else None), n_items, W, cap_items, cap_words,
-                                              _ptr(cursors), _ptr(items), _ptr(keys), d.stream()))
+            if self.umi is None:
+                d.check(d.lib.mirge_shard_scatter(d.ctx, _ptr(src_keys), src_ins, n_items, W, cap_items, cap_words,
+                                                  _ptr(cursors), _ptr(items), _ptr(keys), d.stream()))
+            else:
+                d.check(d.lib.mirge_shard_scatter_centre(d.ctx, _ptr(src_keys), src_ins, n_items, W, self.umi[0], self.umi[1],
+                                                         cap_items, cap_words, _ptr(cursors), _ptr(items), _ptr(keys), d.stream()))
         d.launches += 1
         return {"items": items, "keys": keys, "cursors": cursors, "cap_items": cap_items, "cap_words": cap_words, "br": br}
 
@@ -360,8 +369,34 @@ class ShardedCollapse:
         table.ctrl[0:1].fill_(at)
         return d.empty(n_it, torch.int64), table.arena[a0:at], bases
 
+    def copies_keys(self, table) -> bool:
+        """Whether a round's keys are received into a buffer of their own instead of the end of ``table``'s arena: when
+        repeats dominate the table (its last insert created few keys, DigestEngine.INPLACE_MIN_NEW), so the arena grows
+        with unique sequences rather than with every received key.  (A table that does not count its new keys -- the
+        CPU stand-ins -- keeps the in-place receive.)"""
+        frac = getattr(table, "new_frac", None)
+        return frac is not None and frac < self.eng.INPLACE_MIN_NEW
+
+    def place_copy(self, recv_items, recv_words):
+        """Room for the received keys outside the owner's arena: (items buffer, key buffer, key bases counted from 0)."""
+        d = self.dev
+        n_it, n_w = int(sum(recv_items)), int(sum(recv_words))
+        bases, at = [], 0
+        for w in recv_words:
+            bases.append(at)
+            at += int(w)
+        return d.empty(n_it, torch.int64), d.empty(n_w, torch.int32)[:n_w], bases
+
     def insert(self, table, items, recv_items, bases, local_br=None):
         """The received items into the owner's table (keys already in its arena)."""
+        self._insert(table, items, recv_items, bases, None, local_br)
+
+    def insert_copy(self, table, items, recv_items, bases, keys, local_br=None):
+        """The received items into the owner's table, their keys in ``keys`` (place_copy): only keys new to the table
+        are copied into its arena."""
+        self._insert(table, items, recv_items, bases, keys, local_br)
+
+    def _insert(self, table, items, recv_items, bases, keys, local_br):
         import ctypes as C
 
         from .device import _ptr
@@ -380,10 +415,14 @@ class ShardedCollapse:
         kb = (C.c_uint64 * W)(*[int(x) for x in bases])
         with d.timed("shard_rebase"):
             d.check(d.lib.mirge_shard_rebase(d.ctx, _ptr(items), W, cnt, kb, d.stream()))
-        table.reserve(n, 0)
+        n_words = 0 if keys is None else int(keys.numel())
+        if n_words and table.arena_used + n_words > table.arena.numel() and self.comm is not None:
+            self.comm.synchronize()  # the arena is about to move: nothing may still be arriving in the old one
+        table.reserve(n, n_words)
         scratch = d.empty(2 * n, torch.int32)
+        src = table.arena if keys is None else keys
         with d.timed("collapse"):
-            d.check(d.lib.mirge_collapse_insert_list(d.ctx, C.byref(table.struct), _ptr(table.arena), _ptr(items), n, _ptr(scratch), d.stream()))
+            d.check(d.lib.mirge_collapse_insert_list(d.ctx, C.byref(table.struct), _ptr(src), _ptr(items), n, _ptr(scratch), d.stream()))
         d.launches += 5
         before = table.n_keys
         table.check()
@@ -410,7 +449,11 @@ class ShardedCollapse:
                 self.comm.wait_stream(main)  # (the repeated scatter runs on the launch stream)
         send_it, send_w = self.split_cursors(allc[rank, :W])
         recv_it, recv_w = [int(allc[s, rank]) >> 32 for s in range(W)], [int(allc[s, rank]) & 0xFFFFFFFF for s in range(W)]
-        r_items, r_keys, bases = self.place(table, recv_it, recv_w)
+        copy = self.copies_keys(table)
+        if copy:
+            r_items, r_keys, bases = self.place_copy(recv_it, recv_w)
+        else:
+            r_items, r_keys, bases = self.place(table, recv_it, recv_w)
         ci, cw = packed["cap_items"], packed["cap_words"]
         s_items = [packed["items"][d * ci : d * ci + send_it[d]] for d in range(W)]
         s_keys = [packed["keys"][d * cw : d * cw + send_w[d]] for d in range(W)]
@@ -428,7 +471,7 @@ class ShardedCollapse:
 
         ev = None
         if self._cuda:
-            for t in (packed["items"], packed["keys"], r_items, table.arena):
+            for t in (packed["items"], packed["keys"], r_items, r_keys):
                 t.record_stream(self.comm)
             with torch.cuda.stream(self.comm):
                 with self.dev.timed("shard_a2a"):
@@ -437,7 +480,7 @@ class ShardedCollapse:
                 ev.record(self.comm)
         else:
             wire()
-        r.update(items=r_items, recv_items=recv_it, bases=bases, ev_data=ev, stage=2)
+        r.update(items=r_items, recv_items=recv_it, bases=bases, keys=r_keys if copy else None, ev_data=ev, stage=2)
         return bool(allc[:, W].any())
 
     def _all_to_all(self, outs, ins):
@@ -461,7 +504,10 @@ class ShardedCollapse:
     def _insert_round(self, table, r, on_piece=None):
         if r["ev_data"] is not None:
             torch.cuda.current_stream(self.dev.tdev).wait_event(r["ev_data"])
-        self.insert(table, r["items"], r["recv_items"], r["bases"], r["packed"]["br"])
+        if r["keys"] is None:
+            self.insert(table, r["items"], r["recv_items"], r["bases"], r["packed"]["br"])
+        else:
+            self.insert_copy(table, r["items"], r["recv_items"], r["bases"], r["keys"], r["packed"]["br"])
         if on_piece is not None:
             on_piece(table)
 
@@ -621,11 +667,11 @@ class ExchangeWorker:
 
 # ---------------------------------------------------------------------------------------------------
 # The two entry points for one process per GPU (torchrun): same arguments and, on rank 0, the same return
-# values as digest.baking / manifoldAlign.bwtAlign.  Samples are dealt round-robin to the ranks (a sample's
-# reads -- and with UMIs its first-level table -- stay on one GPU), every sample's unique sequences are
-# hash-partitioned to their owners with one all-to-all, owners keep the per-sample counts of their slice and
-# annotate it against replicated libraries; rank 0 gathers (sequence, counts, annotation) for the DataFrame
-# (SURVEY.md section 8e).
+# values as digest.baking / manifoldAlign.bwtAlign.  Every sample is digested by all ranks at once: the reads of a
+# plain FASTQ file are cut into record-aligned byte ranges that every rank reads itself, a compressed file is read by
+# one rank; either way every batch's keys go to their owners before the collapse (ShardedCollapse).  Owners keep the
+# per-sample counts of their slice and annotate it against replicated libraries; rank 0 gathers (sequence, counts,
+# annotation) for the DataFrame (SURVEY.md section 8e).
 # ---------------------------------------------------------------------------------------------------
 
 _SHARD = {}
@@ -665,9 +711,42 @@ def assemble_table(gathered, names):
     return df, order, offs, int(all_keys.shape[0])
 
 
+def sample_is_splittable(path: str) -> bool:
+    """Whether every rank can read its own share of the file (an uncompressed regular file, ingest.fastq_split_points).
+    A compressed stream cannot be cut: one rank reads it whole."""
+    import os
+
+    from . import ingest
+
+    try:
+        return os.path.isfile(path) and ingest.sniff(path) == "plain"
+    except OSError:  # (fails when the rank that reads it opens it)
+        return False
+
+
+def sample_sources(paths, rank: int, world: int, threads=None):
+    """This rank's input of every sample, in order: (sample index, reader or None).  A plain file: the rank's
+    record-aligned byte range (possibly empty); a compressed file: the whole reader on rank ``s % world`` (read / inflated
+    ahead over that rank's compressed files), None on the others.  Readers are closed by the caller."""
+    from . import ingest
+
+    whole = [not sample_is_splittable(str(p)) for p in paths]
+    mine = [s for s in range(len(paths)) if whole[s] and s % world == rank]
+    with ingest.SampleReadahead([str(paths[s]) for s in mine], threads=threads) as readahead:
+        for s, path in enumerate(paths):
+            if whole[s]:
+                src = readahead.open(mine.index(s)) if s % world == rank else None
+            else:
+                cuts = ingest.fastq_split_points(str(path), world)
+                src = ingest.PlainReader(str(path), threads, start=cuts[rank], stop=cuts[rank + 1])
+            yield s, src
+
+
 def baking_sharded(args, inFileArray, inFileBaseArray, workDir, device=None, count_mode=None, batch_bytes=256 << 20, group=None):
     """Call on every rank.  Returns (complete_set, sampleReadCounts, trimmedReadCounts, trimmedReadCountsUnique);
     complete_set is the DataFrame of digest.baking on rank 0 and None elsewhere."""
+    import os
+
     import numpy as np
 
     from . import digest as DG
@@ -679,41 +758,49 @@ def baking_sharded(args, inFileArray, inFileBaseArray, workDir, device=None, cou
     dev = device or Device(torch.cuda.current_device())
     eng = DigestEngine(dev, cfg)
     umi = cfg.umi()
-    local = CollapseTable(dev, min_keys=1 << 20)
+    dedup = bool(getattr(args, "umiDedup", False))
+    tcf = bool(getattr(args, "tcf_out", False))
     first_level = CollapseTable(dev, min_keys=1 << 20) if umi is not None else None
     owner = CollapseTable(dev, min_keys=1 << 20)
+    target = first_level if umi is not None else owner  # with UMIs the scatter hashes the centre: both levels owner-local
     streamer = DG.HostStreamer(eng, batch_bytes)
+    # (collective: may create communicators.)  With one rank every key is its own: the trim kernels write the keys
+    # straight into the target's arena, as in digest.baking, instead of a batch buffer that is scattered to itself
+    sc = ShardedCollapse(eng, world, group=group, umi=umi) if world > 1 else None
+    tdev = dev.tdev if "nccl" in str(dist.get_backend(group)) else None
     names = list(inFileBaseArray)
     counts_read = np.zeros(len(names), dtype=np.int64)
     per_sample = []  # (owner ids, counts) of this rank's slice, per sample
-    empty = torch.zeros(0, dtype=torch.int32, device=dev.tdev)
-    # this rank's files are read / inflated ahead of the sample it is digesting (ingest.py)
-    mine = [s for s in range(len(inFileArray)) if s % world == rank]
-    readahead = DG.ingest.SampleReadahead([str(inFileArray[s]) for s in mine], threads=DG._host_threads(args))
-    for s, path in enumerate(inFileArray):
-        if s % world == rank:
-            umi_csv = None
-            if umi is not None and getattr(args, "umiDedup", False):
-                import os
-
-                umi_csv = os.path.join(str(workDir), names[s] + "_umiCounts.csv")
-            with readahead.open(mine.index(s)) as f:
-                res = DG.digest_sample(eng, f, local, first_level, bool(getattr(args, "umiDedup", False)), batch_bytes, umi_csv, streamer)
-            counts_read[s] = res.count
-            if getattr(args, "tcf_out", False):
-                # <sample>.trim.collapse.fa (digest.py:226-235) by the rank that digested the sample: its local table
-                # holds exactly the sample's completeDict
-                DG.write_tcf(workDir, names[s], local, res)
-            ids, cnt = res.ids_d, res.counts_d
-        else:
-            ids, cnt = empty, empty
-        exchange_and_merge(dev, local, ids, cnt, owner, world, group=group)  # collective
+    for s, src in sample_sources(list(inFileArray), rank, world, DG._host_threads(args)):
+        try:  # (collective: a rank without input for this sample joins the rounds of the others)
+            counts_read[s] = streamer.run(src if src is not None else DG._BytesSource(b""), target, sharded=sc)
+        finally:
+            if src is not None:
+                src.close()
+        if umi is not None:
+            # digest_sample's second level, on the owner
+            ids1, cnt1 = first_level.drain()
+            DG.umi_collapse(dev, first_level, ids1, cnt1, owner, umi, cfg.minimum_length, dedup)
+            if dedup:
+                keys1 = first_level.export_keys()[ids1.cpu().numpy()]
+                rows = DG.umi_csv_rows(keys1, cnt1.cpu().numpy().astype(np.int64), umi, cfg.minimum_length)
+                got = gather_arrays([np.frombuffer(rows.encode("latin-1"), dtype=np.uint8)], 0, group, tdev)
+                if got is not None:
+                    DG.write_umi_csv_rows(os.path.join(str(workDir), names[s] + "_umiCounts.csv"),
+                                          "".join(g[0].tobytes().decode("latin-1") for g in got))
+            first_level.reset()
         o_ids, o_cnt = owner.drain()
-        per_sample.append((o_ids.cpu().numpy().astype(np.int64), o_cnt.cpu().numpy().astype(np.int64)))
-        local.reset()
-    readahead.close()
-    # counters (digest.py:212-217): records parsed by the digesting rank, emitted counts and unique sequences
-    # summed over the owners
+        ids_h, cnt_h = o_ids.cpu().numpy().astype(np.int64), o_cnt.cpu().numpy().astype(np.int64)
+        per_sample.append((ids_h, cnt_h))
+        if tcf:
+            # <sample>.trim.collapse.fa (digest.py:226-235) at rank 0 from every owner's (sequence, count) pairs
+            got = gather_arrays([owner.export_keys()[ids_h], cnt_h], 0, group, tdev)
+            if got is not None:
+                width = max([g[0].dtype.itemsize for g in got] + [1])
+                DG.write_tcf_rows(workDir, names[s], np.concatenate([g[0].astype("S%d" % width) for g in got]),
+                                  np.concatenate([g[1] for g in got]))
+    # counters (digest.py:212-217): records parsed by every rank, emitted counts and unique sequences summed over the
+    # owners
     tot = torch.zeros((3, len(names)), dtype=torch.int64, device=dev.tdev)
     tot[0] = torch.from_numpy(counts_read).to(dev.tdev)
     tot[1] = torch.tensor([int(c.sum()) for _, c in per_sample], dtype=torch.int64, device=dev.tdev)
@@ -725,7 +812,7 @@ def baking_sharded(args, inFileArray, inFileBaseArray, workDir, device=None, cou
     tru = {n: int(tot_h[2, j]) for j, n in enumerate(names)}
     keys = owner.export_keys()
     # the owners' keys and per-sample (id, count) columns at rank 0 as raw arrays (no pickled rows)
-    flat = gather_arrays([keys] + [a for pair in per_sample for a in pair], 0, group, dev.tdev if "nccl" in str(dist.get_backend(group)) else None)
+    flat = gather_arrays([keys] + [a for pair in per_sample for a in pair], 0, group, tdev)
     gathered = None if flat is None else [(g[0], [(g[1 + 2 * j], g[2 + 2 * j]) for j in range(len(names))]) for g in flat]
     _SHARD.clear()
     _SHARD.update(dev=dev, owner=owner, n_own=int(keys.shape[0]))
