@@ -42,6 +42,10 @@ static int trim_slots_of(const mirge_trim_params *p) {
   return (p->umi_mode != MIRGE_UMI_QIAGEN && p->count_mode == MIRGE_COUNT_HEAD) ? p->n_mods : 1;
 }
 
+// largest cutoff / quality base of the NextSeq and quality modifiers (bases start at 1): what keeps the keys of the
+// quality scans (quality_scan_max) inside an int
+#define QUAL_PARAM_MAX 1000
+
 #define FILL_FAIL(...)                  \
   do {                                  \
     snprintf(err, err_len, __VA_ARGS__); \
@@ -59,6 +63,12 @@ static int fill_dev_params(const mirge_trim_params *p, DevParams &d, int &maxm, 
     d.a[i] = p->mod_a[i];
     d.b[i] = p->mod_b[i];
     d.c[i] = p->mod_c[i];
+    const bool nextseq = d.kind[i] == MIRGE_MOD_NEXTSEQ, quality = d.kind[i] == MIRGE_MOD_QUALITY;
+    const int base = nextseq ? d.b[i] : d.c[i];
+    if ((nextseq || quality) && (d.a[i] < 0 || d.a[i] > QUAL_PARAM_MAX || (quality && (d.b[i] < 0 || d.b[i] > QUAL_PARAM_MAX)) ||
+                                 base < 1 || base > QUAL_PARAM_MAX))
+      FILL_FAIL("%s trimming: quality cutoffs must lie in 0..%d and the quality base in 1..%d", nextseq ? "NextSeq" : "quality",
+                QUAL_PARAM_MAX, QUAL_PARAM_MAX);
   }
   d.n_adapters = p->n_adapters;
   d.times = p->times;
@@ -690,32 +700,108 @@ __device__ __forceinline__ int locate_fast(const int a, const RV read, const int
 
 // ------------------------------------------------------------------ quality trimming --------
 
-__device__ __forceinline__ int nextseq_trim_index(const uint8_t *seq, const uint8_t *qual, int len, int cutoff, int base) {
-  int s = 0, max_qual = 0, max_i = len;
-  for (int i = len - 1; i >= 0; --i) {
-    int q = (int)qual[i] - base;
-    if (seq[i] == 'G') q = cutoff - 1;
-    s += cutoff - q;
-    if (s < 0) break;
-    if (s > max_qual) { max_qual = s; max_i = i; }
+// cutadapt's scans (qualtrim.pyx) add cutoff - (qual[i] - base) to a sum s, stop at the first s < 0 and keep the
+// position of the first strict maximum of s in scan order.  Here every position carries one key k = s * 1024 + x, where
+// x (0..1023) falls by one per byte in scan order: x = i scanning down from len, x = 1022 - i scanning up (x = 1023
+// stands for "before position 0").  Then the first strict maximum is the maximum key, s < 0 exactly when k < 0, and a
+// byte step is k += 1024 * (cutoff + base - qual[i]) - 1.  fill_dev_params bounds cutoff and base to
+// 0..QUAL_PARAM_MAX (base >= 1), so |s| <= 512 * 2000 and every key fits an int.
+//
+// quality_scan_max runs the scan four bytes per step: one aligned 32-bit load per line (funnel-shifted to the group's
+// first byte), the four keys of the group, one sign test for all four; in the group that holds the first negative sum
+// only the keys before it count.  The last len % 4 bytes are scanned byte by byte.  Memory: the word loop reads only aligned words that hold a
+// byte of [0, len) of seq / qual, so it never leaves the 16-byte segments the line occupies -- inside the staging
+// buffer of a CTA, and inside the stream for the kernels that read it from global memory.
+static_assert(MIRGE_MAX_READ_LEN <= 1022, "quality scan keys keep the position in 10 bits");
+
+// 0xFF in every byte of x whose bit 7 is set, 0x00 in the others (PRMT's sign-replicating byte select)
+__device__ __forceinline__ uint32_t byte_msb_mask(uint32_t x) {
+#ifdef ADAPTER_SEARCH_HOST
+  return ((x >> 7) & 0x01010101u) * 0xFFu;
+#else
+  uint32_t r;
+  asm("prmt.b32 %0, %1, 0, 0xBA98;" : "=r"(r) : "r"(x));
+  return r;
+#endif
+}
+
+// qual[i] << 10 of the byte b (0..3) of a group word
+__device__ __forceinline__ int qbyte_k(uint32_t w, int b) { return (int)(((w >> (8 * b)) & 0xFFu) << 10); }
+
+// Largest key of the scan of qual[0, len) (DOWN: from len - 1 to 0, else from 0 to len - 1) that starts at key k.
+// cb = cutoff + base.  NEXTSEQ: positions where seq holds 'G' add 1 to s (qualtrim's q = cutoff - 1).
+template <bool DOWN, bool NEXTSEQ>
+__device__ __forceinline__ int quality_scan_max(const uint8_t *qual, const uint8_t *seq, const int len, const int cb, int k) {
+  const int step = cb * 1024 - 1;
+  int best = k, n = len;  // bytes not scanned yet
+  if (n >= 4) {
+    // a G byte of seq turns into the quality byte cb - 1 (step 1024 - 1).  Clamped to a byte: when cb - 1 > 255 every
+    // byte adds at least 2 to s, G or not, so the scan runs to the end and its result does not depend on the value.
+    const uint32_t g4 = 0x01010101u * (uint32_t)min(cb - 1, 255);
+    // Each step loads the word that holds the group's last byte in scan order (DOWN: byte n - 4, UP: byte len - n + 3);
+    // the word the step before loaded holds its first byte.  The group is funnel_r(loaded, before) scanning down and
+    // funnel_l(before, loaded) scanning up; when the group is word-aligned only the loaded word is used.
+    const int aq = (int)((uintptr_t)qual & 3u), as = NEXTSEQ ? (int)((uintptr_t)seq & 3u) : 0;
+    const uint32_t shq = DOWN ? 8u * (uint32_t)((len + aq) & 3) : 32u - 8u * (uint32_t)aq;
+    const uint32_t shs = DOWN ? 8u * (uint32_t)((len + as) & 3) : 32u - 8u * (uint32_t)as;
+    const uint32_t *qw = (const uint32_t *)(qual - aq), *sw = nullptr;
+    uint32_t q_prev = DOWN ? qw[(len - 1 + aq) >> 2] : qw[0], s_prev = 0;
+    qw += DOWN ? (len - 4 + aq) >> 2 : (3 + aq) >> 2;
+    if (NEXTSEQ) {
+      sw = (const uint32_t *)(seq - as);
+      s_prev = DOWN ? sw[(len - 1 + as) >> 2] : sw[0];
+      sw += DOWN ? (len - 4 + as) >> 2 : (3 + as) >> 2;
+    }
+#pragma unroll 2
+    for (; n >= 4; n -= 4) {
+      const uint32_t qn = *qw, q = DOWN ? __funnelshift_r(qn, q_prev, shq) : __funnelshift_l(q_prev, qn, shq);
+      qw += DOWN ? -1 : 1;
+      q_prev = qn;
+      uint32_t w = q;
+      if (NEXTSEQ) {
+        const uint32_t sn = *sw, s = DOWN ? __funnelshift_r(sn, s_prev, shs) : __funnelshift_l(s_prev, sn, shs);
+        sw += DOWN ? -1 : 1;
+        s_prev = sn;
+        const uint32_t z = s ^ 0x47474747u;  // zero bytes: 'G'
+        const uint32_t not_g = byte_msb_mask(((z & 0x7F7F7F7Fu) + 0x7F7F7F7Fu) | z);
+        w = (q & not_g) | (g4 & ~not_g);
+      }
+      const int k0 = k + step - qbyte_k(w, DOWN ? 3 : 0);
+      const int k1 = k0 + step - qbyte_k(w, DOWN ? 2 : 1);
+      const int k2 = k1 + step - qbyte_k(w, DOWN ? 1 : 2);
+      const int k3 = k2 + step - qbyte_k(w, DOWN ? 0 : 3);
+      if ((k0 | k1 | k2 | k3) < 0) {  // s < 0 in this group: the keys before the first negative one count, then the scan ends
+        if (k0 >= 0) {
+          best = max(best, k0);
+          if (k1 >= 0) {
+            best = max(best, k1);
+            if (k2 >= 0) best = max(best, k2);
+          }
+        }
+        return best;
+      }
+      best = max(best, max(max(k0, k1), max(k2, k3)));
+      k = k3;
+    }
   }
-  return max_i;
+#pragma unroll 1
+  for (; n > 0; --n) {  // the last len % 4 bytes (all of them when len < 4)
+    const int i = DOWN ? n - 1 : len - n;
+    const int d = (NEXTSEQ && seq[i] == 'G') ? 1 : cb - (int)qual[i];
+    k += d * 1024 - 1;
+    if (k < 0) break;
+    best = max(best, k);
+  }
+  return best;
+}
+
+__device__ __forceinline__ int nextseq_trim_index(const uint8_t *seq, const uint8_t *qual, int len, int cutoff, int base) {
+  return quality_scan_max<true, true>(qual, seq, len, cutoff + base, len) & 1023;
 }
 
 __device__ __forceinline__ void quality_trim_index(const uint8_t *qual, int len, int q5, int q3, int base, int &start, int &stop) {
-  int s = 0, max_qual = 0;
-  start = 0; stop = len;
-  for (int i = 0; i < len; ++i) {
-    s += q5 - ((int)qual[i] - base);
-    if (s < 0) break;
-    if (s > max_qual) { max_qual = s; start = i + 1; }
-  }
-  max_qual = 0; s = 0;
-  for (int i = len - 1; i >= 0; --i) {
-    s += q3 - ((int)qual[i] - base);
-    if (s < 0) break;
-    if (s > max_qual) { max_qual = s; stop = i; }
-  }
+  start = 1023 - (quality_scan_max<false, false>(qual, nullptr, len, q5 + base, 1023) & 1023);
+  stop = quality_scan_max<true, false>(qual, nullptr, len, q3 + base, len) & 1023;
   if (start >= stop) { start = 0; stop = 0; }
 }
 

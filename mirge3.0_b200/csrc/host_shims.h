@@ -28,6 +28,10 @@ static inline uint32_t __funnelshift_r(uint32_t lo, uint32_t hi, uint32_t sh) {
   sh &= 31u;
   return sh ? (lo >> sh) | (hi << (32u - sh)) : lo;
 }
+static inline uint32_t __funnelshift_l(uint32_t lo, uint32_t hi, uint32_t sh) {
+  sh &= 31u;
+  return sh ? (hi << sh) | (lo >> (32u - sh)) : hi;
+}
 static inline unsigned __activemask() { return 1u; }
 static inline void __syncwarp(unsigned = 0xffffffffu) {}
 static inline unsigned __ballot_sync(unsigned, bool p) { return p ? 1u : 0u; }

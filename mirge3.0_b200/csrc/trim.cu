@@ -125,26 +125,37 @@ __device__ __forceinline__ int first_adapter_mod() {
 }
 
 // Leftmost p in [start, stop - m] with read[p : p + m] == adapter, or -1.  Pure-ACGT read packed two bits per
-// base (row stride TRIM_THREADS words, zero words after the text), plain adapter of m <= 32 bases in a2.  One
-// funnel shift + compare per position; the upper half is only looked at when the first 16 bases agree.
+// base (row stride TRIM_THREADS words, zero words after the text), plain adapter of m <= 32 bases in a2.  Per word
+// of 16 positions, the positions whose first min(m, 4) bases agree come out of four SWAR compares at once (bit 2s
+// of `cand` for position s: no branch per position); only those are compared in full, lowest first.
 __device__ __forceinline__ int exact_find(const uint32_t *ps, uint64_t a2, int m, int start, int stop) {
   const int last = stop - m;
   if (last < start) return -1;
   const uint32_t a_lo = (uint32_t)a2, a_hi = (uint32_t)(a2 >> 32);
   const uint32_t lo_mask = m >= 16 ? 0xFFFFFFFFu : ((1u << (2 * m)) - 1u);
   const uint32_t hi_mask = m <= 16 ? 0u : (m >= 32 ? 0xFFFFFFFFu : ((1u << (2 * (m - 16))) - 1u));
+  // adapter base k replicated into every 2-bit field (bases past m match anything: 0 fields, and no test)
+  uint32_t rep[4];
+#pragma unroll
+  for (int k = 0; k < 4; ++k) rep[k] = ((a_lo >> (2 * k)) & 3u) * 0x55555555u;
   int wb = start >> 4;
   uint32_t x0 = ps[wb * TRIM_THREADS], x1 = ps[(wb + 1) * TRIM_THREADS], x2 = ps[(wb + 2) * TRIM_THREADS];
 #pragma unroll 1
   for (; 16 * wb <= last; ++wb) {
+    uint32_t cand = 0x55555555u;
 #pragma unroll
-    for (int s = 0; s < 16; ++s) {
-      const uint32_t lo = s ? __funnelshift_r(x0, x1, 2 * s) : x0;
-      if (((lo ^ a_lo) & lo_mask) == 0u) {
-        const uint32_t hi = s ? __funnelshift_r(x1, x2, 2 * s) : x1;
-        const int p = 16 * wb + s;
-        if (((hi ^ a_hi) & hi_mask) == 0u && p >= start && p <= last) return p;
+    for (int k = 0; k < 4; ++k) {
+      if (k < m) {
+        const uint32_t e = (k ? __funnelshift_r(x0, x1, 2 * k) : x0) ^ rep[k];  // zero field: base s + k matches
+        cand &= ~(e | (e >> 1));
       }
+    }
+    while (cand) {
+      const int s = (__ffs((int)cand) - 1) >> 1;
+      cand &= cand - 1u;
+      const uint32_t lo = __funnelshift_r(x0, x1, 2 * s), hi = __funnelshift_r(x1, x2, 2 * s);
+      const int p = 16 * wb + s;
+      if (((lo ^ a_lo) & lo_mask) == 0u && ((hi ^ a_hi) & hi_mask) == 0u && p >= start && p <= last) return p;
     }
     x0 = x1;
     x1 = x2;
