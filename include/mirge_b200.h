@@ -396,6 +396,22 @@ int mirge_sam_format(mirge_ctx *ctx, const mirge_library *lib, const mirge_round
                      const uint64_t *d_name_off, int fill, uint32_t *d_lens, const uint64_t *d_offs, uint8_t *d_out,
                      void *stream);
 
+/* The rows of mapped.csv / unmapped.csv (mirge/__main__.py:164-173), or of baking's complete_set, one per key id
+ * d_rows[i] of table t: the bytes DataFrame.to_csv writes for that row,
+ *   <Sequence>,<annotFlag>,<col 0>,...,<col n_cols-1>,<count 0>,...,<count n_samples-1>\n
+ * Sequence = the key text, quoted as csv.QUOTE_MINIMAL does (in '"' when it holds ',', '"', CR or LF; inner '"' doubled),
+ * bytes >= 0x80 in their two-byte UTF-8 form.  annotFlag = 1 when d_annot[id] != 0xFF.  Column c = the name of reference
+ * MIRGE_HIT_REF(d_hit[id]) of round c when d_annot[id] == c, else empty: the names are finished CSV fields back to back
+ * in d_names, reference r of round c at d_names[d_name_off[d_round_base[c] + r] .. d_name_off[d_round_base[c] + r + 1]).
+ * d_annot = d_hit = NULL: the unannotated form (annotFlag 0, every column empty).  Count s = d_counts[s * count_stride
+ * + id], in decimal.  Two calls: fill = 0 writes d_lens[i] = bytes of row i; after an exclusive scan into d_offs,
+ * fill = 1 writes the rows to d_out + d_offs[i]. */
+int mirge_table_csv_format(mirge_ctx *ctx, const mirge_table *t, const uint32_t *d_rows, uint64_t n, const uint8_t *d_annot,
+                           const uint64_t *d_hit, const uint8_t *d_names, const uint64_t *d_name_off,
+                           const uint32_t *d_round_base, int n_cols, const uint32_t *d_counts, int n_samples,
+                           uint64_t count_stride, int fill, uint32_t *d_lens, const uint64_t *d_offs, uint8_t *d_out,
+                           void *stream);
+
 /* ---- stage 4: counters of annotation.report.csv (summarize, summary.py:692-698,716-770) ---- */
 /* For every (key id, count) pair of ONE sample (the output of mirge_table_drain):
  *   d_round_sum[round of the key] += count            (u64[10]; unannotated keys are skipped)

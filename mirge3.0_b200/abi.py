@@ -173,6 +173,10 @@ SYMBOLS = {
         C.c_int,
         [_P, C.POINTER(Library), C.POINTER(RoundPolicy), C.POINTER(Table), _P, _P, _U64, _P, _P, C.c_int, _P, _P, _P, _P],
     ),
+    "mirge_table_csv_format": (
+        C.c_int,
+        [_P, C.POINTER(Table), _P, _U64, _P, _P, _P, _P, _P, C.c_int, _P, C.c_int, _U64, C.c_int, _P, _P, _P, _P],
+    ),
     "mirge_report_reduce":(C.c_int, [_P, _P, _P, _P, _P, _U64, C.c_uint32, _P, _P, _P, _P]),
     "mirge_annotate_round": (
         C.c_int,

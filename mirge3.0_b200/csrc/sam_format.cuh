@@ -13,33 +13,6 @@
 
 #include "key_format.cuh"
 
-// Output cursor: counts bytes always, stores them only when out != nullptr (the sizing pass).
-struct SamOut {
-  uint8_t *out;
-  uint32_t n;
-  __device__ __forceinline__ void put(uint32_t c) {
-    if (out) out[n] = (uint8_t)c;
-    ++n;
-  }
-  __device__ __forceinline__ void uint(uint32_t v) {  // decimal, most significant digit first (no digit buffer)
-    uint32_t p = 1;
-    while (v / p >= 10u) p *= 10u;
-    for (; p; p /= 10u) put('0' + (v / p) % 10u);
-  }
-  __device__ __forceinline__ void str(const char *s) {
-    while (*s) put((uint32_t)*s++);
-  }
-};
-
-// Byte j of a packed key read left to right: the 2-bit base, or the exception byte stored for j.  Every key writer
-// (mirge_pack_keys, the trim emission, slice_key) lists the exceptions in ascending position, so a cursor that only
-// moves forward finds them; `x` is that cursor, reset to 0 to start over.
-__device__ __forceinline__ uint32_t key_char(const uint32_t *key, int nexc, const uint32_t *exc, int j, int &x) {
-  while (x < nexc && (int)(exc[x] >> 8) < j) ++x;
-  if (x < nexc && (int)(exc[x] >> 8) == j) return exc[x] & 0xFFu;
-  return (uint32_t)"ACGT"[key_base(key, (uint32_t)j)];
-}
-
 // Reference base at library position p: "ACGT" from the 2-bit text, 'N' where the N mask is set (the FASTA's ambiguous
 // bases); positions past the text, which no valid hit reaches, read as 'N' too.
 __device__ __forceinline__ uint32_t sam_ref_char(const mirge_library &lib, uint64_t p) {
@@ -83,7 +56,7 @@ __device__ __forceinline__ uint32_t sam_record(const uint32_t *key, uint64_t h, 
   const uint32_t ref = MIRGE_HIT_REF(h), off = MIRGE_HIT_OFF(h);
   const uint64_t a = (uint64_t)lib.d_ref_off[ref] + off;
   const int seed = pol.seed_len == 0 ? n : min(pol.seed_len, n);
-  SamOut o{out, 0};
+  TextOut o{out, 0};
   int x = 0;
   for (int j = 0; j < len; ++j) o.put(key_char(key, nexc, exc, j, x));  // QNAME: the key text verbatim
   o.str("\t0\t");

@@ -361,6 +361,15 @@ def empty_flag_column(n: int):
     return pd.array(arr, dtype=dt)
 
 
+def sample_columns(table: CollapseTable, samples: List[SampleResult], dtype):
+    """(counts [samples, key ids] on the device, one contiguous row per sample; bool per key id, some sample counted
+    it) from the samples' (key id, count) pairs."""
+    cols_d = torch.zeros((len(samples), int(table.n_keys)), dtype=dtype, device=table.dev.tdev)
+    for j, s in enumerate(samples):
+        cols_d[j, s.ids_d.long()] = s.counts_d.to(dtype)
+    return cols_d, (cols_d != 0).any(dim=0)
+
+
 def build_matrix(table: CollapseTable, samples: List[SampleResult], names: List[str]) -> pd.DataFrame:
     """digest.py:237-261: unique sequences x samples, rows in lexicographic order (what pandas' outer
     join produces for > 1 sample; the single-sample order of the reference is not deterministic).  Columns as the
@@ -370,11 +379,7 @@ def build_matrix(table: CollapseTable, samples: List[SampleResult], names: List[
         8 * n * max(len(samples), 1) <= MATRIX_DEVICE_BYTES
     if on_device:
         # the columns are scattered, selected and ordered on the device; the host sees each of them once, finished
-        tdev = table.dev.tdev
-        cols_d = torch.zeros((len(samples), n), dtype=torch.int64, device=tdev)  # one contiguous row per sample
-        for j, s in enumerate(samples):
-            cols_d[j, s.ids_d.long()] = s.counts_d.long()
-        seen_d = (cols_d != 0).any(dim=0)
+        cols_d, seen_d = sample_columns(table, samples, torch.int64)
         perm_d, offsets_d, data_d = table.export_sorted_device(seen_d)
         order, offsets, data = perm_d.cpu().numpy(), offsets_d.cpu().numpy(), data_d.cpu().numpy()
         del offsets_d, data_d
@@ -409,8 +414,42 @@ def baking(args, inFileArray, inFileBaseArray, workDir, device: Optional[Device]
     """Same contract as the reference ``baking(args, inFileArray, inFileBaseArray, workDir)``:
     returns (complete_set DataFrame, sampleReadCounts, trimmedReadCounts, trimmedReadCountsUnique)."""
     begningTime = time.perf_counter()
-    cfg = P.TrimConfig.from_args(args, count_mode or default_count_mode())
     dev = device or get_device()
+    runlogFile = Path(workDir) / "run.log"
+    outlog = open(str(runlogFile), "a+")
+    quiet = bool(getattr(args, "quiet", False))
+    table, results, umi, sampleReadCounts, trimmedReadCounts, trimmedReadCountsUnique = digest_samples(
+        args, inFileArray, inFileBaseArray, workDir, dev, outlog, quiet, count_mode, batch_bytes)
+    finish3 = time.perf_counter()
+    complete_set = build_matrix(table, results, list(inFileBaseArray))
+    finish4 = time.perf_counter()
+    log_line(outlog, quiet, f"Matrix creation finished in {round(finish4-finish3, 4)} second(s)\n")
+    names = list(inFileBaseArray)
+    _write_histograms(workDir, lambda: _frame_lens(complete_set), lambda j: complete_set[names[j]].to_numpy() > 0, results, names,
+                      umi)
+    EndTime = time.perf_counter()
+    log_line(outlog, quiet, f"Data pre-processing completed in {round(EndTime-begningTime, 4)} second(s)\n",
+             f"\nData pre-processing completed in {round(EndTime-begningTime, 4)} second(s)\n\n")
+    outlog.close()
+    if keep_table:
+        return complete_set, sampleReadCounts, trimmedReadCounts, trimmedReadCountsUnique, table
+    return (complete_set, sampleReadCounts, trimmedReadCounts, trimmedReadCountsUnique)
+
+
+def log_line(outlog, quiet: bool, screen: str, file: Optional[str] = None):
+    """One progress line: print(screen) unless -quiet; ``file`` to run.log as it is (default: ``screen`` ending in one
+    newline)."""
+    if not quiet:
+        print(screen)
+    outlog.write(screen.rstrip("\n") + "\n" if file is None else file)
+
+
+def digest_samples(args, inFileArray, inFileBaseArray, workDir, dev: Device, outlog, quiet: bool, count_mode: Optional[str] = None,
+                   batch_bytes: int = DEFAULT_BATCH_BYTES):
+    """baking()'s per-sample loop (digest.py:133-235): every file digested into one table, the counters, the -tcf /
+    -umi -udd side files and the per-sample log lines.  Returns (table, [SampleResult], umi, sampleReadCounts,
+    trimmedReadCounts, trimmedReadCountsUnique)."""
+    cfg = P.TrimConfig.from_args(args, count_mode or default_count_mode())
     eng = DigestEngine(dev, cfg)
     umi = cfg.umi()
     table = CollapseTable(dev, min_keys=1 << 20)
@@ -420,9 +459,6 @@ def baking(args, inFileArray, inFileBaseArray, workDir, device: Optional[Device]
     trimmedReadCounts: Dict[str, int] = {}
     trimmedReadCountsUnique: Dict[str, int] = {}
     results: List[SampleResult] = []
-    runlogFile = Path(workDir) / "run.log"
-    outlog = open(str(runlogFile), "a+")
-    quiet = bool(getattr(args, "quiet", False))
     # the files of the run are read (and inflated) ahead of the sample being digested, on args.threads workers
     readahead = ingest.SampleReadahead([str(p) for p in inFileArray], threads=_host_threads(args))
     for index, FQfile in enumerate(inFileArray):
@@ -440,31 +476,13 @@ def baking(args, inFileArray, inFileBaseArray, workDir, device: Optional[Device]
         trimmedReadCounts[base] = res.trimmed
         trimmedReadCountsUnique[base] = res.unique
         finish2 = time.perf_counter()
-        if not quiet:
-            print(f"Cutadapt finished for file {base} in {round(finish2-start, 4)} second(s)")
-        outlog.write(f"Cutadapt finished for file {base} in {round(finish2-start, 4)} second(s)\n")
+        log_line(outlog, quiet, f"Cutadapt finished for file {base} in {round(finish2-start, 4)} second(s)")
         if getattr(args, "tcf_out", False):
             write_tcf(workDir, base, table, res)
         finish3 = time.perf_counter()
-        if not quiet:
-            print(f"Collapsing finished for file {base} in {round(finish3-finish2, 4)} second(s)\n")
-        outlog.write(f"Collapsing finished for file {base} in {round(finish3-finish2, 4)} second(s)\n")
+        log_line(outlog, quiet, f"Collapsing finished for file {base} in {round(finish3-finish2, 4)} second(s)\n")
     readahead.close()
-    finish3 = time.perf_counter()
-    complete_set = build_matrix(table, results, list(inFileBaseArray))
-    finish4 = time.perf_counter()
-    if not quiet:
-        print(f"Matrix creation finished in {round(finish4-finish3, 4)} second(s)\n")
-    outlog.write(f"Matrix creation finished in {round(finish4-finish3, 4)} second(s)\n")
-    _write_histograms(workDir, complete_set, results, list(inFileBaseArray), umi)
-    EndTime = time.perf_counter()
-    if not quiet:
-        print(f"Data pre-processing completed in {round(EndTime-begningTime, 4)} second(s)\n")
-    outlog.write(f"\nData pre-processing completed in {round(EndTime-begningTime, 4)} second(s)\n\n")
-    outlog.close()
-    if keep_table:
-        return complete_set, sampleReadCounts, trimmedReadCounts, trimmedReadCountsUnique, table
-    return (complete_set, sampleReadCounts, trimmedReadCounts, trimmedReadCountsUnique)
+    return table, results, umi, sampleReadCounts, trimmedReadCounts, trimmedReadCountsUnique
 
 
 def write_tcf(workDir, base, table: CollapseTable, res: SampleResult):
@@ -482,21 +500,28 @@ def write_tcf_rows(workDir, base, keys: np.ndarray, counts: np.ndarray):
             fo.write(keys[j].decode("latin-1") + "\n")
 
 
-def _write_histograms(workDir, df: pd.DataFrame, results: List[SampleResult], names: List[str], umi):
+def _frame_lens(df: pd.DataFrame) -> np.ndarray:
+    """Text length of every row of a frame from build_matrix (the export's offsets), else of its index."""
+    cached = df.attrs.get("_mirge_b200_keys")
+    if cached is not None and cached.offsets is not None and len(cached.offsets) == len(df) + 1:
+        return cached.lens
+    return df.index.str.len().to_numpy()
+
+
+def _write_histograms(workDir, lens, present, results: List[SampleResult], names: List[str], umi):
     """index_data.js read-length / UMI histograms (digest.py:270-295) through the reference's own
-    FormatJS when miRge is importable.  Deviation (DESIGN.md): the reference appends one length per
-    *chunk-unique* key (digest.py:146-157), which depends on its 4 MB chunk boundaries; here every
-    sample-unique key contributes once."""
+    FormatJS when miRge is importable.  ``lens()``: the text length of every row of the table; ``present(j)``: bool
+    per row, sample j counted it (both called only when the histograms are written).  Deviation (DESIGN.md): the
+    reference appends one length per *chunk-unique* key (digest.py:146-157), which depends on its 4 MB chunk boundaries;
+    here every sample-unique key contributes once."""
     try:
         from mirge.classes.exportHTML import FormatJS  # the reference's visualisation writer
     except Exception:
         return
     histData = FormatJS(workDir)
-    cached = df.attrs.get("_mirge_b200_keys")
-    lens = cached.lens if cached is not None and cached.offsets is not None and len(cached.offsets) == len(df) + 1 else \
-        df.index.str.len().to_numpy()
+    lens = lens()
     for div_idnum, (name, res) in enumerate(zip(names, results), 1):
-        val = lens[df[name].to_numpy() > 0]
+        val = lens[present(div_idnum - 1)]
         if val.size == 0:
             continue
         maxVal, minVal = int(val.max()), int(val.min())

@@ -825,7 +825,8 @@ def baking_sharded(args, inFileArray, inFileBaseArray, workDir, device=None, cou
     class _NoHist:
         hist = np.zeros(0, dtype=np.int64)
 
-    DG._write_histograms(workDir, df, [_NoHist()] * len(names), names, None)
+    DG._write_histograms(workDir, lambda: DG._frame_lens(df), lambda j: df[names[j]].to_numpy() > 0, [_NoHist()] * len(names), names,
+                         None)
     return df, src, trc, tru
 
 

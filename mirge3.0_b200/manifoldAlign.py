@@ -380,6 +380,21 @@ def write_round_sam(path, dev: Device, lib, pol, keys: KeySet, ids: np.ndarray, 
     return n_rec, n_bytes
 
 
+def write_sam_files(args, workDir, dev: Device, libs, keys: KeySet, annot: np.ndarray, key_of_row: Optional[np.ndarray],
+                    hit_of_key: torch.Tensor, spike: bool):
+    """The per-round SAM files for bamFmt.bow2bam (-bam) and the tRF block of summarize (-trf) that ``args`` asks for:
+    records in the order bowtie prints them (input order = table order, round_sam_pairs inside a sequence), formatted
+    on the device.  annot: annotation round of every table row; key_of_row: key id of every row (None: row = key id);
+    hit_of_key: hit word of every key id, on the device."""
+    pols = round_policies()
+    for rnd, fname in sam_rounds(args, spike):
+        rows = np.nonzero(annot == rnd)[0]
+        if rows.size == 0:
+            continue
+        ids = rows if key_of_row is None else key_of_row[rows]
+        write_round_sam(Path(workDir) / fname, dev, libs[ROUND_LIBS[rnd]], pols[rnd], keys, ids, hit_of_key)
+
+
 def _filled_column(old: "pd.Series", rows: np.ndarray, names: np.ndarray, ref: np.ndarray):
     """The annotation column of a round: names[ref] at ``rows``, the old values elsewhere (manifoldAlign.py:17-18,55).
     A column that is still all '' -- what baking() hands over -- is built from codes + dictionary (Arrow dictionary
@@ -539,15 +554,7 @@ def bwtAlign(args, pdDataFrame, workDir, ref_db, libraries: Optional[LibrarySet]
     flag = pdDataFrame[colnames[0]].to_numpy(copy=True)
     flag[annot != 0xFF] = 1
     pdDataFrame[colnames[0]] = flag
-    # per-round SAM files for bamFmt.bow2bam (-bam) and the tRF block of summarize (-trf): records in the order
-    # bowtie prints them (input order = table order, round_sam_pairs inside a sequence), formatted on the device
-    pols = round_policies()
-    for rnd, fname in sam_rounds(args, spike):
-        rows = np.nonzero(annot == rnd)[0]
-        if rows.size == 0:
-            continue
-        ids = rows if key_of_row is None else key_of_row[rows]
-        write_round_sam(Path(workDir) / fname, dev, libs[ROUND_LIBS[rnd]], pols[rnd], keys, ids, hit_of_key)
+    write_sam_files(args, workDir, dev, libs, keys, annot, key_of_row, hit_of_key, spike)
     finish = time.perf_counter()
     if not spike:
         pdDataFrame = pdDataFrame.drop(columns=["spike-in"])

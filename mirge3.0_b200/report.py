@@ -171,20 +171,41 @@ def annotation_report(args, workDir, ref_db, base_names: Sequence[str], pdDataFr
     spike = bool(getattr(args, "spikeIn", False))
     annot, hit = codes_from_dataframe(pdDataFrame, libs, spike)
     n = len(pdDataFrame)
-    mir = libs["mirna"]
     annot_d = torch.from_numpy(annot).to(dev.tdev)
     hit_d = torch.from_numpy(hit).to(dev.tdev)
     ids_d = torch.arange(n, dtype=torch.int32, device=dev.tdev)
-    sums = []
+    samples = []
     for name in base_names:
         col = pdDataFrame[name].to_numpy()
         if n and int(col.max()) >= (1 << 31):
             raise MirgeError("report: a per-sequence count exceeds int32")
+        samples.append((ids_d, torch.from_numpy(col.astype(np.int32)).to(dev.tdev)))
+    return annotation_report_device(args, workDir, ref_db, base_names, annot_d, hit_d, samples, sampleReadCounts, trimmedReadCounts,
+                                    trimmedReadCountsUnique, libraries=libs, device=dev, write=write)
+
+
+def annotation_report_device(args, workDir, ref_db, base_names: Sequence[str], annot_d: torch.Tensor, hit_d: torch.Tensor, samples,
+                             sampleReadCounts, trimmedReadCounts, trimmedReadCountsUnique, rows_d: Optional[torch.Tensor] = None,
+                             libraries: Optional[LibrarySet] = None, device: Optional[Device] = None, write: bool = True):
+    """annotation_report from device arrays instead of a DataFrame: annot_d (uint8) / hit_d (int64), the annotation
+    round and hit word of every key id; ``samples``, each sample's (key ids int32, counts int32) on the device, taken
+    as they are (annotation_report checks a DataFrame's counts against 2^31 before it calls this; a table's drained
+    counts are int32 already); ``rows_d``, the key ids of the table's rows (None: every key id is a row).  Returns the
+    three DataFrames."""
+    from .manifoldAlign import get_device, load_libraries
+
+    dev = device or get_device()
+    libs = libraries or load_libraries(args, ref_db, dev)
+    spike = bool(getattr(args, "spikeIn", False))
+    mir = libs["mirna"]
+    sums = []
+    for ids_d, cnt_d in samples:
         ss = SampleSums(dev, mir.n_refs)
-        ss.add(annot_d, hit_d, ids_d, torch.from_numpy(col.astype(np.int32)).to(dev.tdev))
+        ss.add(annot_d, hit_d, ids_d, cnt_d)
         sums.append(ss.host())
+    a, h = (annot_d, hit_d) if rows_d is None else (annot_d[rows_d], hit_d[rows_d])
     has_exact = np.zeros(mir.n_refs, dtype=bool)
-    has_exact[(hit[annot == 0] >> 28) & 0xFFFFFFF] = True
+    has_exact[((h[a == 0] >> 28) & 0xFFFFFFF).cpu().numpy()] = True
     mfname = str(args.organism_name) + "_merges_" + str(ref_db) + ".csv"
     member, merged = read_merges(Path(args.libraries_path) / args.organism_name / "annotation.Libs" / mfname)
     summary, mir_counts, mir_rpm = build_report(base_names, sums, has_exact, mir.names, member, merged, sampleReadCounts,
